@@ -3,7 +3,7 @@
 1,000 synthetic haplotypes x 10,000 SNPs, 69-state decoding quantities; every pair is decoded over the whole sequence and
 IBD segments with per-segment age estimates are called, as FastSMC::run does with hashing off).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the whole job (499,500 haplotype pairs x 10,000 sites).
   value : pair-sites/s with the pair list resident in HBM (fsmc_plan_launch only inside the timed region)
@@ -17,12 +17,18 @@ data set dealt to the N ranks from a shared counter, files to .ibd.gz, host and 
 
 --impl reference times the CPU restatement of the reference algorithm (oracle/, multi-threaded over batches, AVX2 lane
 vectorisation like the reference's SIMD build) on a bounded sample of the same workload on the host cores.
+
+--dump-outputs DIR writes the segment records of the last timed step of the headline run to DIR/segment_<field>.npy (see
+dump_segments), so that two builds can be compared output for output on the same seeded inputs.
+
+Data sets and output files go to a per-user directory under the system's temporary directory (WORK), never into the tree.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -41,10 +47,12 @@ NCU_DRAM_BYTES_PER_PAIR_SITE = (109.922461e9 + 109.458343e9) / (37888 * 10000)  
 # over cfg2 (blocks of 128 sites); refineKernel adds 75.8 GB per step (profiles/r2_final_refine_ncu_full.txt)
 NCU_SPARSE_DRAM_BYTES_PER_PAIR_SITE = (87.827249e9 + 101.530119e9) / (499500 * 10000)
 WORKLOAD = "cfg2: all-pairs, hashing off, 1000 haplotypes x 10000 SNPs, S=69 (30-100-2000), time=50, batchSize=32"
+# per user: files another user's run left in a shared directory could not be overwritten
+WORK = os.path.join(tempfile.gettempdir(), f"fsmc_bench_{os.getuid()}")
 
 
 def dataset_root(rank):
-    return f"/tmp/fsmc_bench/r{rank}/cfg2_{N_HAPS}x{N_SITES}"
+    return f"{WORK}/r{rank}/cfg2_{N_HAPS}x{N_SITES}"
 
 
 def make_dataset(rank):
@@ -147,7 +155,7 @@ def reference_sample(cores):
     # concurrent processes carry equal work and the slowest one does not understate the CPU rate
     off_diagonal = [j for j in range(1, REF_JOBS + 1) if int(j ** 0.5) ** 2 != j]
     for k in range(cores):
-        argv = pyoracle.reference_command("avx", root, DQ, f"/tmp/fsmc_bench/ref_out_{k}", hashing=0, jobs=REF_JOBS,
+        argv = pyoracle.reference_command("avx", root, DQ, f"{WORK}/ref_out_{k}", hashing=0, jobs=REF_JOBS,
                                           jobInd=off_diagonal[k % len(off_diagonal)], time=50, noConditionalAgeEstimates=1,
                                           batchSize=32)
         procs.append(subprocess.Popen(argv, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True))
@@ -168,7 +176,7 @@ def port_sample(cores, n_pairs):
     pyoracle.build()
     _declare_sample(pyoracle)
     root = make_dataset(0)
-    o = pyoracle.Oracle(root, DQ, "/tmp/fsmc_bench/ref_out", hashing=False, time=50, noConditionalAgeEstimates=True,
+    o = pyoracle.Oracle(root, DQ, f"{WORK}/ref_out", hashing=False, time=50, noConditionalAgeEstimates=True,
                         doPerPairMAP=True, doPerPairPosteriorMean=True, batchSize=32)
     t0 = time.time()
     ps = pyoracle.lib().fo_decode_sample(o._h, n_pairs, cores)
@@ -206,6 +214,20 @@ def cpu_baseline():
             "per_thread": ps / dt / cores}
 
 
+def dump_segments(directory, segments, tiles, prefix=""):
+    """The segment records that a caller of the timed path receives, one DIR/<prefix>segment_<field>.npy per field, in the
+    records' order (pair row, start site): the haplotype pair of the record's row (hapA, hapB), its sites and its level as
+    float64 (exact), its scores (prob, postMean, mapTime) as the float32 the kernels write.  cfg2 gives ~4.6e5 records,
+    ~28 MB in all."""
+    os.makedirs(directory, exist_ok=True)
+    row = segments["pair"].astype(np.int64)
+    fields = {"hapA": tiles["hapA"].reshape(-1)[row], "hapB": tiles["hapB"].reshape(-1)[row]}
+    fields.update({f: segments[f] for f in ("posStart", "posEnd", "mapState", "level", "prob", "postMean", "mapTime")})
+    for name, v in fields.items():
+        np.save(os.path.join(directory, f"{prefix}segment_{name}.npy"),
+                v.astype(np.float32 if v.dtype == np.float32 else np.float64))
+
+
 def max_over_ranks(value, world, device="cuda"):
     """Step time of the job = the slowest rank's (the only cross-rank operation of the benchmark)."""
     if world == 1:
@@ -239,15 +261,15 @@ def jobs_run(asmc, rank, world, local, dist):
     rank, and the host/kernel seconds per rank that explain it."""
     import torch
     from fastsmc_b200 import synth
-    root = f"/tmp/fsmc_bench/cfg4s_{JOBS_SAMPLES}x{JOBS_SITES}"
+    root = f"{WORK}/cfg4s_{JOBS_SAMPLES}x{JOBS_SITES}"
     if rank == 0 and not os.path.exists(root + ".hap.gz"):
         synth.dataset(root, 2 * JOBS_SAMPLES, JOBS_SITES, JOBS_SPAN_BP, JOBS_CHROM, SEED + 2)
     if dist:
         dist.barrier()
     p = asmc.DecodingParams()
     p.verbose = False
-    p.inFileRoot, p.decodingQuantFile, p.outFileRoot = root, DQ, f"/tmp/fsmc_bench/jobs_out/r{rank}"
-    os.makedirs("/tmp/fsmc_bench/jobs_out", exist_ok=True)
+    p.inFileRoot, p.decodingQuantFile, p.outFileRoot = root, DQ, f"{WORK}/jobs_out/r{rank}"
+    os.makedirs(f"{WORK}/jobs_out", exist_ok=True)
     p.decodingModeString, p.foldData, p.usingCSFS = "array", True, True
     p.FastSMC, p.hashing, p.batchSize, p.time, p.min_m = True, True, 32, 50, 1.5
     p.doPerPairMAP = p.doPerPairPosteriorMean = p.outputIbdSegmentLength = True
@@ -323,7 +345,12 @@ def main():
     ap.add_argument("--no-e2e-run", action="store_true", help="skip the one-off FastSMC.run() wall-clock measurement")
     ap.add_argument("--no-jobs-run", action="store_true", help="skip the jobs/jobInd-partitioned hashing run (jobs_run)")
     ap.add_argument("--no-states159", action="store_true", help="skip the 159-state legs (state-split kernels)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the segment records of the headline run's last timed step to DIR/segment_<field>.npy "
+                         "(rank<r>_segment_<field>.npy per rank under torchrun)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -347,7 +374,7 @@ def main():
     root = dataset_root(0)
     p = asmc.DecodingParams()
     p.verbose = False
-    p.inFileRoot, p.decodingQuantFile, p.outFileRoot = root, DQ, f"/tmp/fsmc_bench/r{rank}/out"
+    p.inFileRoot, p.decodingQuantFile, p.outFileRoot = root, DQ, f"{WORK}/r{rank}/out"
     p.decodingModeString, p.foldData, p.usingCSFS = "array", True, True
     p.FastSMC, p.hashing, p.batchSize, p.time = True, False, 32, 50
     p.noConditionalAgeEstimates = p.doPerPairMAP = p.doPerPairPosteriorMean = p.outputIbdSegmentLength = True
@@ -418,6 +445,8 @@ def main():
     clocks = ClockSampler(local)
     rank0_ms, results = timed_steps(lanes, clocks)
     r = results[0]
+    if args.dump_outputs:
+        dump_segments(args.dump_outputs, r.segments, tiles, f"rank{rank}_" if world > 1 else "")
     per_step = [rank0_ms / args.steps]
     n_segments = int(r.stats.numSegments)
     scratch_bytes = int(r.stats.scratchBytes)
@@ -467,7 +496,7 @@ def main():
             pl.launch()
             torch.cuda.synchronize()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            n159 = max(1, min(3, args.steps))
+            n159 = args.steps
             e0.record(st159)
             for _ in range(n159):
                 pl.launch()

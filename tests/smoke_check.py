@@ -1,4 +1,7 @@
 """smoke(): one small invocation of the CUDA hot path on cuda:0, checked against the CPU oracle (test infrastructure)."""
+import os
+import tempfile
+
 import numpy as np
 
 from conftest import FASTSMC_EXAMPLE, FASTSMC_EXAMPLE_DQ, REGRESSION_PARAMS, context_from_oracle
@@ -7,8 +10,9 @@ from conftest import FASTSMC_EXAMPLE, FASTSMC_EXAMPLE_DQ, REGRESSION_PARAMS, con
 def run(verbose=False):
     from fastsmc_b200 import _native as N
     from oracle import pyoracle
-    o = pyoracle.Oracle(FASTSMC_EXAMPLE, FASTSMC_EXAMPLE_DQ, "/tmp/fsmc_smoke", hashing=True, **REGRESSION_PARAMS)
-    n = o.run("/tmp/fsmc_smoke_oracle.ibd.gz")
+    with tempfile.TemporaryDirectory() as tmp:
+        o = pyoracle.Oracle(FASTSMC_EXAMPLE, FASTSMC_EXAMPLE_DQ, os.path.join(tmp, "o"), hashing=True, **REGRESSION_PARAMS)
+        n = o.run(os.path.join(tmp, "oracle.ibd.gz"))
     ints, floats = o.segments()
     batches, cands = o.batches(), o.candidates()
     ctx = context_from_oracle(o, pyoracle)

@@ -99,12 +99,12 @@ def _oracle_segments(o):
 
 
 @pytest.mark.parametrize("hashing", [True, False])
-def test_segments_exact_mode_identical_to_oracle(oracle_mod, hashing):
+def test_segments_exact_mode_identical_to_oracle(oracle_mod, tmp_path, hashing):
     """Whole-job segment lists (golden G1 / G2 configurations): identical records in identical order."""
     from fastsmc_b200 import _native as N
     extra = dict(hashing=True) if hashing else dict(hashing=False, jobInd=7, jobs=9)
     o = oracle_mod.Oracle(FASTSMC_EXAMPLE, FASTSMC_EXAMPLE_DQ, "/tmp/fsmc_test", **extra, **REGRESSION_PARAMS)
-    n = o.run("/tmp/fsmc_test_oracle.ibd.gz")
+    n = o.run(str(tmp_path / "oracle.ibd.gz"))
     ints, floats = o.segments()
     batches = o.batches()
     ctx = context_from_oracle(o, oracle_mod)
@@ -127,10 +127,10 @@ def test_segments_exact_mode_identical_to_oracle(oracle_mod, hashing):
     assert np.array_equal(seg["mapTime"].view(np.uint32), floats[:, 2].copy().view(np.uint32))
 
 
-def test_segments_fast_mode_matches_oracle_within_tolerance(oracle_mod):
+def test_segments_fast_mode_matches_oracle_within_tolerance(oracle_mod, tmp_path):
     from fastsmc_b200 import _native as N
     o = oracle_mod.Oracle(FASTSMC_EXAMPLE, FASTSMC_EXAMPLE_DQ, "/tmp/fsmc_test", hashing=True, **REGRESSION_PARAMS)
-    n = o.run("/tmp/fsmc_test_oracle.ibd.gz")
+    n = o.run(str(tmp_path / "oracle.ibd.gz"))
     ints, floats = o.segments()
     batches = o.batches()
     cands = o.candidates()
@@ -149,12 +149,12 @@ def test_segments_fast_mode_matches_oracle_within_tolerance(oracle_mod):
     assert (seg["mapState"] != ints[:, 6]).mean() < 5e-3
 
 
-def test_no_hashing_job_exact(oracle_mod):
+def test_no_hashing_job_exact(oracle_mod, tmp_path):
     """Golden G2 configuration (hashing off, job 7 of 9): all-pairs tiles over the whole sequence."""
     from fastsmc_b200 import _native as N
     o = oracle_mod.Oracle(FASTSMC_EXAMPLE, FASTSMC_EXAMPLE_DQ, "/tmp/fsmc_test", hashing=False, jobInd=7, jobs=9,
                           **REGRESSION_PARAMS)
-    n = o.run("/tmp/fsmc_test_oracle_nohash.ibd.gz")
+    n = o.run(str(tmp_path / "oracle.ibd.gz"))
     ints, floats = o.segments()
     # pair stream: first record of each (batch, lane) is enough to recover hapA/hapB only for pairs with
     # segments, so re-enumerate the job's pairs exactly as HMM::decodeAll does (HMM.cpp:311-357)
@@ -231,12 +231,12 @@ def test_fast_kernel_per_site_outputs_69_states(synthetic69, split):
         assert (r.site_map[rows, :to - frm] != mp).mean() < 2e-3
 
 
-def test_fast_kernel_segments_69_states(synthetic69, split):
+def test_fast_kernel_segments_69_states(synthetic69, tmp_path, split):
     """Whole all-pairs job slice through the production kernel vs the oracle: same segments (a boundary may move only
     where the IBD probability is within tolerance of a threshold), sums and age estimates within 1e-4."""
     from fastsmc_b200 import _native as N
     o, ctx = synthetic69
-    n = o.run("/tmp/fsmc_test69_oracle.ibd.gz")
+    n = o.run(str(tmp_path / "oracle.ibd.gz"))
     ints, floats = o.segments()
     H = o.num_haps
     a, b = [], []
@@ -325,7 +325,7 @@ def test_narrow_kernel_matches_oracle_and_wide_kernel(oracle_mod, synthetic69, s
 
 
 @pytest.mark.parametrize("time", [50, 100, 140], ids=["time50-2quads", "time100-3quads", "time140-4quads"])
-def test_lane_split_kernels_159_states(oracle_mod, time):
+def test_lane_split_kernels_159_states(oracle_mod, tmp_path, time):
     """FastSMC's default flags on the example data (age estimates conditional on TMRCA < time) at 159 states: the lane-split
     kernels (decode_lane.cuh; records, and full beta rows with FSMC_WIDE_KERNEL) vs the oracle: same segments, per-segment
     values and per-site IBD probability within 1e-4, over ragged windows, a partially filled tile and a one-site window."""
@@ -333,7 +333,7 @@ def test_lane_split_kernels_159_states(oracle_mod, time):
     params = dict(REGRESSION_PARAMS, noConditionalAgeEstimates=False, time=time)  # records of 2, 3 and 4 quads
     o = oracle_mod.Oracle(FASTSMC_EXAMPLE, FASTSMC_EXAMPLE_DQ, "/tmp/fsmc_test159n", hashing=True, **params)
     assert o.age_threshold == o.state_threshold == time // 10
-    n = o.run("/tmp/fsmc_test159n_oracle.ibd.gz")
+    n = o.run(str(tmp_path / "oracle.ibd.gz"))
     ints, floats = o.segments()
     batches = o.batches()
     cands = o.candidates()
@@ -397,13 +397,13 @@ def _seg_key(s):
     return (int(s["pair"]), int(s["posStart"]), int(s["posEnd"]))
 
 
-def test_sparse_age_estimates_match_oracle_and_dense_kernel(synthetic69, monkeypatch):
+def test_sparse_age_estimates_match_oracle_and_dense_kernel(synthetic69, tmp_path, monkeypatch):
     """noConditionalAgeEstimates on whole-chromosome windows: narrow sweeps + checkpoints + refinement inside the IBD runs
     (sparseKernel) vs the oracle (1e-4) and vs the kernel that streams every beta row through HBM (same segments)."""
     from conftest import check_segments_up_to_threshold_ties
     from fastsmc_b200 import _native as N
     o, ctx = synthetic69
-    n = o.run("/tmp/fsmc_test69_oracle.ibd.gz")
+    n = o.run(str(tmp_path / "oracle.ibd.gz"))
     ints, floats = o.segments()
     a, b = _all_pairs(o.num_haps)
     tiles = ctx.make_tiles(a, b, sites=o.sites)
