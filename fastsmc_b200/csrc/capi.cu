@@ -134,6 +134,7 @@ struct fsmc_ctx {
   fsmc::DeviceModel kernelModel{};
   DevBuf<float> kernelSiteRows;
   DevBuf<float> laneAux;  // kernelModel.laneAux
+  DevBuf<float> bwdRows;  // kernelModel.bwdRows
   DevBuf<float> siteRows, prior, expTimes, colRatios;
   DevBuf<uint64_t> haps;
   long long numHaps = 0;
@@ -326,7 +327,7 @@ FastChoice chooseFastKernel(const DeviceModel& m, const unsigned flags, const bo
   if (sparse) {
     const int rq = (m.stateThreshold + 1 + 3) / 4;
     FastKernelFn fn = rq == 1   ? fsmc::decodeNarrowKernel<69, 1, 4, kFastDepth, 128, 2, 1>
-                      : rq == 2 ? fsmc::decodeNarrowKernel<69, 2, 4, kFastDepth, 128, 2, 1>
+                      : rq == 2 ? fsmc::decodeNarrowKernel<69, 2, 2, kFastDepth, 128, 2, 1>
                       : rq == 3 ? fsmc::decodeNarrowKernel<69, 3, 2, kFastDepth, 128, 2, 1>
                                 : fsmc::decodeNarrowKernel<69, 4, 2, kFastDepth, 128, 2, 1>;
     if (const char* e = std::getenv("FSMC_SPARSE_VARIANT")) {  // development: A/B of code-size variants
@@ -340,9 +341,9 @@ FastChoice chooseFastKernel(const DeviceModel& m, const unsigned flags, const bo
   if (S == 69 && narrow) {
     // 2 CTAs x 4 warps per SM at 255 registers: measured 12.2e9 pair-sites/s vs 10.1e9 at 3 CTAs / 168 registers (spills)
     const int rq = (m.stateThreshold + 1 + 3) / 4;
-    // ring slots hold 4 window positions when two CTAs of that size fit an SM (records of up to 8 floats), else 2
+    // ring slots hold 4 window positions when two CTAs of that size fit an SM (records of 4 floats), else 2
     FastKernelFn fn = rq == 1   ? fsmc::decodeNarrowKernel<69, 1, 4, kFastDepth, 128, 2>
-                      : rq == 2 ? fsmc::decodeNarrowKernel<69, 2, 4, kFastDepth, 128, 2>
+                      : rq == 2 ? fsmc::decodeNarrowKernel<69, 2, 2, kFastDepth, 128, 2>
                       : rq == 3 ? fsmc::decodeNarrowKernel<69, 3, 2, kFastDepth, 128, 2>
                                 : fsmc::decodeNarrowKernel<69, 4, 2, kFastDepth, 128, 2>;
     if (const char* e = std::getenv("FSMC_SPARSE_VARIANT")) {
@@ -371,8 +372,8 @@ size_t fastSmemBytes(const FastChoice& fc, const int S)
   }
   const size_t warps = fc.threads / 32;
   if (fc.narrow) {
-    const size_t group = fc.recordQuads <= 2 ? 4 : 2;
-    const size_t slot = group * static_cast<size_t>(fsmc::kRowArrays) * fc.Spad * 4 + (group + 1) * static_cast<size_t>(fc.recordQuads) * 32 * 16;
+    const size_t group = fc.recordQuads == 1 ? 4 : 2;
+    const size_t slot = group * static_cast<size_t>(fsmc::kBwdArrays) * fc.Spad * 4 + (group + 1) * static_cast<size_t>(fc.recordQuads) * 32 * 16;
     return warps * kFastDepth * slot + warps * kFastDepth * sizeof(uint64_t);
   }
   return warps * (kFastDepth * (static_cast<size_t>(fc.Spad) * 32 * 4 + static_cast<size_t>(fsmc::kRowArrays) * fc.Spad * 4) +
@@ -591,6 +592,15 @@ int fsmc_set_model(fsmc_ctx* ctx, const fsmc_model* mdl)
   }
   ctx->model.laneAux = nullptr;
   ctx->kernelModel.laneAux = nullptr;
+  ctx->model.bwdRows = nullptr;
+  ctx->kernelModel.bwdRows = nullptr;
+  if (ctx->kernelModel.S == 69) {
+    FSMC_CUDA(ctx->bwdRows.ensure(static_cast<size_t>(L) * fsmc::kBwdArrays * ctx->kernelModel.Spad));
+    fsmc::buildBackwardRowsKernel<<<blocks, threads, 0, st>>>(ctx->kernelModel.Spad, L, ctx->kernelModel.siteRows, ctx->bwdRows.p);
+    FSMC_CUDA(cudaGetLastError());
+    FSMC_CUDA(cudaStreamSynchronize(st));
+    ctx->kernelModel.bwdRows = ctx->bwdRows.p;
+  }
   if (ctx->kernelModel.S == 159) {
     FSMC_CUDA(ctx->laneAux.ensure(static_cast<size_t>(L) * fsmc::laneAuxFloats159()));
     fsmc::buildLaneAux159(L, ctx->kernelModel.siteRows, ctx->laneAux.p, blocks, st);

@@ -354,6 +354,109 @@ __device__ __forceinline__ float forwardStep(const float* colRatios, float (&x)[
   return run;
 }
 
+// ---- the backward step on the narrow kernel's backward rows (buildBackwardRowsKernel) -----------------------------------
+// The emission is part of the coefficients, so the packed multiply v = beta * E per pair of states goes: 7 issue slots and
+// 4 LDS.128 per two states instead of 8 and 5.  Same phases and chains as backwardStep; the products round differently
+// ((U E) x instead of U (E x): fp32, within the fast mode's 1e-4).
+// x: beta(p+1) on entry (kept); y: unscaled beta(p) on return.  row = backward row of site p+1.
+template <int S>
+__device__ __forceinline__ void backwardStepFolded(const float (&x)[S], float (&y)[S], const float* row, const int cls)
+{
+  constexpr int SQ = (S + 3) / 4, Spad = SQ * 4, QM = (SQ + 1) / 2;
+  static_assert(4 * QM < S - 1, "the lower half lies below the last state");
+  const float4* UsE = reinterpret_cast<const float4*>(row + cls * Spad);  // Us[k] E[k] = U[k-1] E[k]
+  const float4* DE = reinterpret_cast<const float4*>(row + (3 + cls) * Spad);
+  const float4* BE = reinterpret_cast<const float4*>(row + (6 + cls) * Spad);
+  const float4* Rr = reinterpret_cast<const float4*>(row + 9 * Spad);
+  float bu = 0.f, bl = 0.f;
+  float above = 0.f;  // U[k] E[k+1] x[k+1] for the state k the BU chain reaches next
+  // phase A
+#pragma unroll
+  for (int i = 0; i < QM; ++i) {
+    const int qu = SQ - 1 - i;
+    if (qu >= QM) {
+      const float4 u4 = UsE[qu], r4 = Rr[qu];
+#pragma unroll
+      for (int jp = 1; jp >= 0; --jp) {
+        const int k = 4 * qu + 2 * jp, k1 = k + 1;
+        if (k1 < S) {
+          const float2 t = __fmul2_rn(pk(f4(u4, 2 * jp), f4(u4, 2 * jp + 1)), pk(x[k], x[k1]));
+          if (k1 == S - 1) {
+            y[k1] = 0.f;  // BU[S-1] = 0
+          } else {
+            bu = fmaf(f4(r4, 2 * jp + 1), bu, above);  // BU[k] = U[k] E[k+1] x[k+1] + RR[k] BU[k+1]
+            y[k1] = bu;
+          }
+          bu = fmaf(f4(r4, 2 * jp), bu, t.y);
+          y[k] = bu;
+          above = t.x;
+        } else if (k < S) {
+          above = f4(u4, 2 * jp) * x[k];
+          if (k == S - 1) {
+            y[k] = 0.f;
+          } else {
+            bu = fmaf(f4(r4, 2 * jp), bu, above);
+            y[k] = bu;
+          }
+        }
+      }
+    }
+    {
+      const int ql = i;
+      const float4 d4 = DE[ql], b4 = BE[ql];
+#pragma unroll
+      for (int jp = 0; jp < 2; ++jp) {
+        const int k = 4 * ql + 2 * jp, k1 = k + 1;
+        const float bl0 = bl;
+        const float bl1 = fmaf(f4(b4, 2 * jp), x[k], bl0);  // BL[k+1] = BL[k] + B[k] E[k] x[k]
+        bl = fmaf(f4(b4, 2 * jp + 1), x[k1], bl1);
+        const float2 w = __ffma2_rn(pk(f4(d4, 2 * jp), f4(d4, 2 * jp + 1)), pk(x[k], x[k1]), pk(bl0, bl1));
+        y[k] = w.x;
+        y[k1] = w.y;
+      }
+    }
+  }
+  // phase B
+#pragma unroll
+  for (int i = 0; i < QM; ++i) {
+    {
+      const int ql = QM - 1 - i;
+      const float4 u4 = UsE[ql], r4 = Rr[ql];
+#pragma unroll
+      for (int jp = 1; jp >= 0; --jp) {
+        const int k = 4 * ql + 2 * jp, k1 = k + 1;
+        const float2 t = __fmul2_rn(pk(f4(u4, 2 * jp), f4(u4, 2 * jp + 1)), pk(x[k], x[k1]));
+        const float b1 = fmaf(f4(r4, 2 * jp + 1), bu, above);
+        const float b0 = fmaf(f4(r4, 2 * jp), b1, t.y);
+        bu = b0;
+        above = t.x;
+        const float2 w = __fadd2_rn(pk(y[k], y[k1]), pk(b0, b1));
+        y[k] = w.x;
+        y[k1] = w.y;
+      }
+    }
+    const int qu = QM + i;
+    if (qu < SQ) {
+      const float4 d4 = DE[qu], b4 = BE[qu];
+#pragma unroll
+      for (int jp = 0; jp < 2; ++jp) {
+        const int k = 4 * qu + 2 * jp, k1 = k + 1;
+        if (k1 < S) {
+          const float bl0 = bl;
+          const float bl1 = fmaf(f4(b4, 2 * jp), x[k], bl0);
+          bl = fmaf(f4(b4, 2 * jp + 1), x[k1], bl1);
+          const float2 w = __fadd2_rn(__ffma2_rn(pk(f4(d4, 2 * jp), f4(d4, 2 * jp + 1)), pk(x[k], x[k1]), pk(bl0, bl1)),
+                                      pk(y[k], y[k1]));
+          y[k] = w.x;
+          y[k1] = w.y;
+        } else if (k < S) {
+          y[k] = fmaf(f4(d4, 2 * jp), x[k], bl) + y[k];
+        }
+      }
+    }
+  }
+}
+
 // One item per lane with `pred` (decode_sparse.cuh): slots from one atomic per warp, the descriptor, and alpha at the block's
 // first site (copied from the warp's scratch, column `lane`).  Returns the lane's new chain head.  Out of line on purpose:
 // it runs at a few percent of the sites, and inlined into the unrolled site loop it slowed every site down (the loop no
@@ -402,11 +505,12 @@ static __device__ __noinline__ int emitSparseItems(SparseItem* items, float* ite
 constexpr int kNarrowMaxQuads = 4;  // record = up to 16 floats: sT <= 15
 constexpr int kNarrowGroup = 4;     // window positions per ring slot (one bulk copy and one barrier per group)
 
-// Ring slot of one warp: G coefficient rows followed by G+1 records (the extra record is the all-ones beta of the
-// window's last site, which rides with the first group of the backward sweep).
+// Ring slot of one warp: G coefficient rows (backward rows in the backward sweep, the smaller 8-array rows in the forward
+// sweep) followed by G+1 records (the extra record is the all-ones beta of the window's last site, which rides with the
+// first group of the backward sweep).  RQ = 1, G = 4: 112.7 KB per CTA of 4 warps at DEPTH 2, two CTAs per SM.
 template <int S_T, int RQ, int G> struct NarrowSlot {
   static constexpr int SQ = (S_T + 3) / 4, Spad = SQ * 4;
-  static constexpr uint32_t kCoefBytes = kRowArrays * Spad * 4;
+  static constexpr uint32_t kCoefBytes = kBwdArrays * Spad * 4;
   static constexpr uint32_t kRecBytes = RQ * 32 * 16;
   static constexpr uint32_t kBytes = G * kCoefBytes + (G + 1) * kRecBytes;
 };
@@ -442,7 +546,9 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const 
   constexpr uint32_t kRecBytes = Slot::kRecBytes;
   constexpr uint32_t kCoefBytes = Slot::kCoefBytes;
   constexpr size_t kRecFloats = static_cast<size_t>(RQ) * 32 * 4;
-  constexpr size_t kRowFloats = static_cast<size_t>(kRowArrays) * Spad;
+  constexpr size_t kRowFloats = static_cast<size_t>(kRowArrays) * Spad;  // forward sweep: the 8-array rows
+  constexpr uint32_t kRowBytes = static_cast<uint32_t>(kRowFloats) * 4;
+  constexpr size_t kBwdFloats = static_cast<size_t>(kBwdArrays) * Spad;  // backward sweep: the folded rows
   constexpr int kWarps = THREADS / 32;
   constexpr size_t kWarpBytes = static_cast<size_t>(DEPTH) * Slot::kBytes;
   static_assert(S >= 4 * kNarrowMaxQuads && RQ >= 1 && RQ <= kNarrowMaxQuads, "record quads index the state vector");
@@ -549,7 +655,7 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const 
           const int slot = g % DEPTH;
           const uint32_t bytes = static_cast<uint32_t>(j1 - j0) * kCoefBytes;
           mbarExpectTx(&bars[slot], bytes);
-          bulkLoad(coefArea(slot), rowBase + static_cast<size_t>(len - j1) * kRowFloats, bytes, &bars[slot]);
+          bulkLoad(coefArea(slot), m.bwdRows + static_cast<size_t>(from + len - j1) * kBwdFloats, bytes, &bars[slot]);
         }
       };
       for (int g = 0; g < DEPTH && g < nGroups; ++g) {
@@ -596,7 +702,7 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const 
         auto step = [&](const int i, float (&x)[S], float (&y)[S], const bool rescale) {
           const int p = len - 2 - (j0 + i);
           const int cls = bits.cls(from + p + 1);
-          backwardStep<S>(x, y, coef + static_cast<size_t>(n - 1 - i) * kRowFloats, cls);
+          backwardStepFolded<S>(x, y, coef + static_cast<size_t>(n - 1 - i) * kBwdFloats, cls);
           float divisor = 1.0f;
           if (rescale) {
             divisor = sumStates<S>(y);
@@ -659,8 +765,8 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const 
           const int p0 = g * G;
           const uint32_t n = static_cast<uint32_t>(min(G, len - p0));
           const int slot = g % DEPTH;
-          mbarExpectTx(&bars[slot], n * (kCoefBytes + kRecBytes));
-          bulkLoad(coefArea(slot), rowBase + static_cast<size_t>(p0) * kRowFloats, n * kCoefBytes, &bars[slot]);
+          mbarExpectTx(&bars[slot], n * (kRowBytes + kRecBytes));
+          bulkLoad(coefArea(slot), rowBase + static_cast<size_t>(p0) * kRowFloats, n * kRowBytes, &bars[slot]);
           bulkLoad(recArea(slot), slab + static_cast<size_t>(p0) * kRecFloats, n * kRecBytes, &bars[slot]);
         }
       };

@@ -29,6 +29,7 @@ namespace fsmc
 {
 
 constexpr int kRowArrays = 8;  // per-site table row: E_homMajor, E_het, E_homMinor, D, B, U, RR, U shifted by one state (each Spad floats)
+constexpr int kBwdArrays = 10;  // per-site backward row of the narrow kernel, emission folded in (buildBackwardRowsKernel)
 constexpr unsigned kFull = 0xffffffffu;
 
 struct DeviceModel {
@@ -36,6 +37,7 @@ struct DeviceModel {
   int Spad;    // S rounded up to a multiple of 4 (float4 loads)
   int L;       // sites
   const float* siteRows;   // [L][kRowArrays][Spad]
+  const float* bwdRows;    // [L][kBwdArrays][Spad] backward rows with the emission folded in; 69-state models only
   const float* laneAux;    // [L][Spad + 16] suffix products of RR inside the state quarters (decode_lane.cuh); 159-state models only
   const float* prior;      // [Spad] initialStateProb
   const float* expTimes;   // [Spad] expectedTimes
@@ -666,6 +668,31 @@ static __global__ void buildSiteRowsKernel(const int S, const int Spad, const in
     for (int j = 0; j < kRowArrays; ++j) {
       out[static_cast<size_t>(j) * Spad] = v[j];
     }
+  }
+}
+
+// The narrow kernel's backward rows (decode_fast.cuh), from the rows above: the emission of each genotype class c is
+// multiplied into the coefficients once per site, so that the backward step never multiplies beta by it.
+//   backward row of site s: [UsE_0..2 | DE_0..2 | BE_0..2 | RR],  UsE_c = Us_s E_s[c], DE_c = D_s E_s[c], BE_c = B_s E_s[c]
+static __global__ void buildBackwardRowsKernel(const int Spad, const int L, const float* __restrict__ rows,
+                                               float* __restrict__ bwd)
+{
+  const long long total = static_cast<long long>(L) * Spad;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const int site = static_cast<int>(i / Spad);
+    const int k = static_cast<int>(i % Spad);
+    const float* r = rows + static_cast<size_t>(site) * kRowArrays * Spad + k;
+    const float D = r[3 * Spad], B = r[4 * Spad], Us = r[7 * Spad];
+    float* b = bwd + static_cast<size_t>(site) * kBwdArrays * Spad + k;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      const float e = r[c * Spad];
+      b[c * Spad] = __fmul_rn(Us, e);
+      b[(3 + c) * Spad] = __fmul_rn(D, e);
+      b[(6 + c) * Spad] = __fmul_rn(B, e);
+    }
+    b[9 * Spad] = r[6 * Spad];  // RR
   }
 }
 
