@@ -67,6 +67,15 @@ class Stats(C.Structure):
         ("kernelLaunches", C.c_int32), ("statesKernel", C.c_int32), ("scratchBytes", C.c_int64),
         ("narrowKernel", C.c_int32), ("tileWarps", C.c_int32),
         ("sparseKernel", C.c_int32), ("checkpointSites", C.c_int32), ("sparseItems", C.c_int64), ("checkpointBytes", C.c_int64),
+        ("d2hBytes", C.c_int64),
+    ]
+
+
+class DeviceOutputs(C.Structure):
+    _fields_ = [
+        ("laneRow", C.c_void_p), ("numRows", C.c_int64), ("siteStride", C.c_int64),
+        ("siteMean_dev", C.c_void_p), ("siteMap_dev", C.c_void_p), ("siteIbd_dev", C.c_void_p),
+        ("sitePosterior_dev", C.c_void_p), ("sumPosterior_dev", C.c_void_p), ("stateWeight", C.c_void_p),
     ]
 
 
@@ -79,6 +88,7 @@ EXPORTS = [
     "fsmc_last_error", "fsmc_version", "fsmc_device_count", "fsmc_ctx_create", "fsmc_ctx_destroy",
     "fsmc_ctx_set_stream", "fsmc_set_model", "fsmc_set_haplotypes", "fsmc_decode", "fsmc_plan_create",
     "fsmc_plan_launch", "fsmc_plan_collect", "fsmc_plan_destroy", "fsmc_seed", "fsmc_query_kernel",
+    "fsmc_decode_device", "fsmc_column_min_f32", "fsmc_column_min_i32",
 ]
 
 _lib = None
@@ -103,6 +113,9 @@ def lib():
         L.fsmc_plan_launch.argtypes = [C.c_void_p, C.c_void_p]
         L.fsmc_plan_collect.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Request), C.POINTER(Stats)]
         L.fsmc_plan_destroy.argtypes = [C.c_void_p, C.c_void_p]
+        L.fsmc_decode_device.argtypes = [C.c_void_p, C.POINTER(Request), C.POINTER(DeviceOutputs), C.POINTER(Stats)]
+        for f in (L.fsmc_column_min_f32, L.fsmc_column_min_i32):
+            f.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]
         _lib = L
     return _lib
 
@@ -268,6 +281,42 @@ class Context:
                 continue
             seg = out["seg"][:stats.numSegments] if out["seg"] is not None else None
             return DecodeResult(seg, out["mean"], out["smap"], out["ibd"], stats, out["post"], out["psum"])
+
+    # ---- device-resident outputs (torch tensors or anything with data_ptr() on this context's device)
+    def decode_device(self, tiles, flags, lane_row, num_rows, site_stride, *, site_mean=None, site_map=None, site_ibd=None,
+                      site_posterior=None, sum_posterior=None, state_weight=None):
+        """fsmc_decode_device: the kernels write the given device buffers, row lane_row[tile*32+lane] of each.  The buffers'
+        sizes are checked here (the C ABI sees raw pointers); where they lie is checked by the library."""
+        T = len(tiles["tilePairs"])
+        per_pair = site_stride * num_rows
+        need = {"site_mean": (site_mean, per_pair), "site_map": (site_map, per_pair), "site_ibd": (site_ibd, per_pair),
+                "site_posterior": (site_posterior, per_pair * self.states),
+                "sum_posterior": (sum_posterior, (3 if flags & SUM_BY_GENOTYPE else 1) * self.states * self.sites)}
+        for name, (t, n) in need.items():
+            if t is not None and t.numel() < n:
+                raise FastSMCError(-1, f"{name} has {t.numel()} elements, {n} needed")
+            if t is not None and not t.is_contiguous():
+                raise FastSMCError(-1, f"{name} is not contiguous")
+        rows = np.ascontiguousarray(lane_row, dtype=np.int64)
+        assert rows.shape == (T * TILE,)
+        w = _f32(state_weight) if state_weight is not None else None
+        req = Request(T, _p(tiles["hapA"]), _p(tiles["hapB"]), _p(tiles["tilePairs"]), _p(tiles["tileFrom"]),
+                      _p(tiles["tileTo"]), _p(tiles["tileScanFrom"]), _p(tiles["tileScanTo"]), flags,
+                      None, 0, None, None, None, 0, None, None)
+        ptr = lambda t: t.data_ptr() if t is not None else None  # noqa: E731
+        out = DeviceOutputs(_p(rows), int(num_rows), int(site_stride), ptr(site_mean), ptr(site_map), ptr(site_ibd),
+                            ptr(site_posterior), ptr(sum_posterior), _p(w))
+        stats = Stats()
+        _check(lib().fsmc_decode_device(self._h, C.byref(req), C.byref(out), C.byref(stats)))
+        return stats
+
+    def column_min(self, m, out_min, out_argmin):
+        """fsmc_column_min_f32 / _i32 of a 2-D row-major device tensor (float32 or int32) on the context's stream."""
+        if m.dim() != 2 or m.stride(1) != 1 or out_min.numel() < m.shape[1] or out_argmin.numel() < m.shape[1]:
+            raise FastSMCError(-1, "column_min: needs a row-major 2-D matrix and outputs of one value per column")
+        rows, cols = m.shape
+        f = lib().fsmc_column_min_f32 if m.dtype.is_floating_point else lib().fsmc_column_min_i32
+        _check(f(self._h, m.data_ptr(), rows, cols, m.stride(0), out_min.data_ptr(), out_argmin.data_ptr()))
 
     # ---- split phase (device-resident inputs)
     def plan(self, tiles, flags, segment_capacity=1 << 20, site_stride=0):

@@ -16,6 +16,7 @@
 #include <thread>
 #include <vector>
 
+#include "column_min.cuh"
 #include "decode_kernels.cuh"
 #include "decode_fast.cuh"
 #include "decode_sparse.cuh"
@@ -174,6 +175,7 @@ struct fsmc_ctx {
   // (kernel, threads, dynamic shared memory) -> resident CTAs per SM: the attribute / occupancy queries of a plan are made
   // once per context, not once per call (they and cudaMemGetInfo were 10-90 ms of a 300 ms fsmc_decode call)
   std::map<std::tuple<const void*, int, size_t>, int> occupancy;
+  DevBuf<uint32_t> colMinPart;  // fsmc_column_min_*: per-chunk (value, row) of every column
 };
 
 struct fsmc_plan {
@@ -218,6 +220,14 @@ struct fsmc_plan {
   size_t sortTempBytes = 0;
   int refineBlocks = 0;
   size_t refineSmem = 0;
+  // fsmc_decode_device: the kernels write the caller's device buffers at the rows of laneRow
+  bool deviceOut = false;
+  std::vector<uint32_t> hostLaneRow;
+  std::vector<float> hostWeight;
+  DevBuf<uint32_t> laneRow;
+  DevBuf<float> stateWeight;  // [S]: the caller's weights, or ones
+  float *outMean = nullptr, *outIbd = nullptr, *outPosterior = nullptr, *outSum = nullptr;
+  int* outMap = nullptr;
 };
 
 namespace
@@ -677,7 +687,29 @@ cudaError_t residentBlocks(fsmc_ctx* ctx, const void* fn, const int threads, con
 }
 }  // namespace
 
-int fsmc_plan_create(fsmc_ctx* ctx, const fsmc_decode_request* req, fsmc_plan** out)
+namespace
+{
+// memory of the context's device (cudaMalloc'd or managed), not host memory or another device's
+int checkDevicePtr(const fsmc_ctx* ctx, const void* p, const char* what)
+{
+  cudaPointerAttributes at{};
+  const cudaError_t e = cudaPointerGetAttributes(&at, p);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(FSMC_E_INVALID, "%s is not a CUDA pointer (%s)", what, cudaGetErrorString(e));
+  }
+  if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) {
+    return fail(FSMC_E_INVALID, "fsmc_decode_device: %s is host memory, device memory of device %d is needed", what, ctx->device);
+  }
+  if (at.device != ctx->device) {
+    return fail(FSMC_E_INVALID, "fsmc_decode_device: %s is on device %d, the context on device %d", what, at.device, ctx->device);
+  }
+  return FSMC_OK;
+}
+}  // namespace
+
+// fsmc_plan_create; with `dev`, the outputs are the caller's device buffers (fsmc_decode_device) and none is allocated
+static int planCreate(fsmc_ctx* ctx, const fsmc_decode_request* req, const fsmc_device_outputs* dev, fsmc_plan** out)
 {
   if (!ctx || !req || !out) {
     return fail(FSMC_E_INVALID, "fsmc_plan_create: NULL argument");
@@ -734,9 +766,52 @@ int fsmc_plan_create(fsmc_ctx* ctx, const fsmc_decode_request* req, fsmc_plan** 
     pairSites += static_cast<double>(n) * (e - f);
     scanSites += seg ? static_cast<double>(req->tileScanTo[t] - req->tileScanFrom[t]) : 0.0;
   }
-  if (siteOut && req->siteStride < maxLen) {
-    return fail(FSMC_E_INVALID, "fsmc_plan_create: siteStride=%lld < longest window %lld",
-                static_cast<long long>(req->siteStride), maxLen);
+  const long long siteStride = dev ? dev->siteStride : req->siteStride;
+  if (siteOut && siteStride < maxLen) {
+    return fail(FSMC_E_INVALID, "fsmc_plan_create: siteStride=%lld < longest window %lld", siteStride, maxLen);
+  }
+  if (dev) {
+    if (seg) {
+      return fail(FSMC_E_INVALID, "fsmc_decode_device: FSMC_CALL_SEGMENTS is not supported (segments go to the host: fsmc_decode)");
+    }
+    if (dev->numRows < 1 || dev->numRows > 0x7fffffffll) {
+      return fail(FSMC_E_INVALID, "fsmc_decode_device: numRows=%lld out of range [1, 2^31)", static_cast<long long>(dev->numRows));
+    }
+    const struct {
+      unsigned flag;
+      const void* p;
+      const char* name;
+    } outs[] = {{FSMC_SITE_MEAN, dev->siteMean_dev, "siteMean_dev"},
+                {FSMC_SITE_MAP, dev->siteMap_dev, "siteMap_dev"},
+                {FSMC_SITE_IBD, dev->siteIbd_dev, "siteIbd_dev"},
+                {FSMC_SITE_POSTERIOR, dev->sitePosterior_dev, "sitePosterior_dev"},
+                {FSMC_SUM_POSTERIOR, dev->sumPosterior_dev, "sumPosterior_dev"}};
+    for (const auto& o : outs) {
+      if (!(flags & o.flag)) {
+        continue;
+      }
+      if (!o.p) {
+        return fail(FSMC_E_INVALID, "fsmc_decode_device: %s is NULL but its flag is set", o.name);
+      }
+      const int rc = checkDevicePtr(ctx, o.p, o.name);
+      if (rc != FSMC_OK) {
+        return rc;
+      }
+    }
+    if (siteOut && T > 0) {
+      if (!dev->laneRow) {
+        return fail(FSMC_E_INVALID, "fsmc_decode_device: laneRow is NULL");
+      }
+      for (long long t = 0; t < T; ++t) {
+        for (int l = 0; l < req->tilePairs[t]; ++l) {
+          const int64_t r = dev->laneRow[t * 32 + l];
+          if (r < 0 || r >= dev->numRows) {
+            return fail(FSMC_E_INVALID, "fsmc_decode_device: laneRow[%lld]=%lld outside [0, numRows=%lld)", t * 32 + l,
+                        static_cast<long long>(r), static_cast<long long>(dev->numRows));
+          }
+        }
+      }
+    }
   }
   if (seg && req->segmentCapacity < 0) {
     return fail(FSMC_E_INVALID, "fsmc_plan_create: negative segmentCapacity");
@@ -762,7 +837,8 @@ int fsmc_plan_create(fsmc_ctx* ctx, const fsmc_decode_request* req, fsmc_plan** 
   plan->maxLen = maxLen;
   plan->pairSites = pairSites;
   plan->segmentCapacity = seg ? req->segmentCapacity : 0;
-  plan->siteStride = siteOut ? req->siteStride : 0;
+  plan->siteStride = siteOut ? siteStride : 0;
+  plan->deviceOut = dev != nullptr;
 
   // longest-window-first launch order (dynamic queue → LPT schedule); stable, so equal windows keep input order
   std::vector<int>& order = plan->hostOrder;
@@ -800,19 +876,43 @@ int fsmc_plan_create(fsmc_ctx* ctx, const fsmc_decode_request* req, fsmc_plan** 
     }
   }
   const size_t nSite = nLane * static_cast<size_t>(plan->siteStride);
-  if (flags & FSMC_SITE_MEAN) {
+  if (dev) {
+    plan->outMean = dev->siteMean_dev;
+    plan->outMap = dev->siteMap_dev;
+    plan->outIbd = dev->siteIbd_dev;
+    plan->outPosterior = dev->sitePosterior_dev;
+    plan->outSum = dev->sumPosterior_dev;
+    plan->hostLaneRow.assign(nLane, 0u);
+    if (siteOut) {
+      for (long long t = 0; t < T; ++t) {
+        for (int l = 0; l < req->tilePairs[t]; ++l) {
+          plan->hostLaneRow[t * 32 + l] = static_cast<uint32_t>(dev->laneRow[t * 32 + l]);
+        }
+      }
+    }
+    plan->hostWeight.assign(m.S, 1.f);
+    if (dev->stateWeight) {
+      std::copy(dev->stateWeight, dev->stateWeight + m.S, plan->hostWeight.begin());
+    }
+    FSMC_CUDA(plan->laneRow.ensure(nLane));
+    FSMC_CUDA(plan->stateWeight.ensure(m.S));
+    if (T > 0) {
+      FSMC_CUDA(cudaMemcpyAsync(plan->laneRow.p, plan->hostLaneRow.data(), nLane * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    }
+    FSMC_CUDA(cudaMemcpyAsync(plan->stateWeight.p, plan->hostWeight.data(), m.S * sizeof(float), cudaMemcpyHostToDevice, st));
+  } else if (flags & FSMC_SITE_MEAN) {
     FSMC_CUDA(plan->siteMean.ensure(nSite));
   }
-  if (flags & FSMC_SITE_MAP) {
+  if (!dev && (flags & FSMC_SITE_MAP)) {
     FSMC_CUDA(plan->siteMap.ensure(nSite));
   }
-  if (flags & FSMC_SITE_IBD) {
+  if (!dev && (flags & FSMC_SITE_IBD)) {
     FSMC_CUDA(plan->siteIbd.ensure(nSite));
   }
-  if (flags & FSMC_SITE_POSTERIOR) {
+  if (!dev && (flags & FSMC_SITE_POSTERIOR)) {
     FSMC_CUDA(plan->sitePosterior.ensure(nSite * static_cast<size_t>(ctx->model.S)));
   }
-  if (flags & FSMC_SUM_POSTERIOR) {
+  if (!dev && (flags & FSMC_SUM_POSTERIOR)) {
     FSMC_CUDA(plan->sumPosterior.ensure(sumPosteriorCount(ctx->model, flags)));
   }
   plan->launched = false;
@@ -832,6 +932,10 @@ int fsmc_plan_create(fsmc_ctx* ctx, const fsmc_decode_request* req, fsmc_plan** 
   plan->narrow = fc.narrow;
   plan->tileWarps = fc.splitWarps > 0 ? fc.splitWarps : 1;
   plan->mode = kc.mode;
+  if (dev && (fc.narrow || fc.sparse)) {
+    return fail(FSMC_E_INVALID, "fsmc_decode_device: flags 0x%x run a narrow kernel, which has no caller rows: set FSMC_SITE_MEAN, "
+                "FSMC_SITE_MAP or FSMC_WIDE_KERNEL", flags);
+  }
   // tiles in flight per CTA: one per warp, except for the state-split kernels (one tile per CTA)
   int warpsPerBlock = fc.splitWarps > 0 ? 1 : (plan->fast ? fc.threads : kc.threads) / 32;
   const size_t smemLimit = ctx->prop.sharedMemPerBlockOptin;
@@ -973,6 +1077,11 @@ int fsmc_plan_create(fsmc_ctx* ctx, const fsmc_decode_request* req, fsmc_plan** 
   return FSMC_OK;
 }
 
+int fsmc_plan_create(fsmc_ctx* ctx, const fsmc_decode_request* req, fsmc_plan** out)
+{
+  return planCreate(ctx, req, nullptr, out);
+}
+
 namespace
 {
 // item buffers of a sparse plan, (re)sized to plan->itemCapacity
@@ -1035,15 +1144,20 @@ int fsmc_plan_launch(fsmc_ctx* ctx, fsmc_plan* plan)
     a.segments = plan->segments.p;
     a.segmentCount = plan->counters.p;
     a.segmentCapacity = plan->segmentCapacity;
-    a.siteMean = plan->siteMean.p;
-    a.siteMap = plan->siteMap.p;
-    a.siteIbd = plan->siteIbd.p;
-    a.sitePosterior = plan->sitePosterior.p;
-    a.sumPosterior = plan->sumPosterior.p;
+    const bool dev = plan->deviceOut;
+    a.siteMean = dev ? plan->outMean : plan->siteMean.p;
+    a.siteMap = dev ? plan->outMap : plan->siteMap.p;
+    a.siteIbd = dev ? plan->outIbd : plan->siteIbd.p;
+    a.sitePosterior = dev ? plan->outPosterior : plan->sitePosterior.p;
+    a.sumPosterior = dev ? plan->outSum : plan->sumPosterior.p;
+    a.laneRow = dev ? plan->laneRow.p : nullptr;
+    a.stateWeight = dev ? plan->stateWeight.p : nullptr;
     const int sumPlanes = (plan->flags & FSMC_SUM_BY_GENOTYPE) ? 3 : 1;
     const int sumWarps = plan->blocks * plan->tilesPerBlock;
     if (plan->flags & FSMC_SUM_POSTERIOR) {
-      FSMC_CUDA(cudaMemsetAsync(plan->sumPosterior.p, 0, sumPosteriorCount(ctx->model, plan->flags) * sizeof(float), st));
+      if (!dev) {  // the caller's sums are added to
+        FSMC_CUDA(cudaMemsetAsync(plan->sumPosterior.p, 0, sumPosteriorCount(ctx->model, plan->flags) * sizeof(float), st));
+      }
       if (plan->sumOnFast) {
         a.sumScratch = ctx->sumScratch.p;
         FSMC_CUDA(cudaMemsetAsync(ctx->sumScratch.p, 0, static_cast<size_t>(sumWarps) * sumPlanes * m.L * m.Spad * sizeof(float), st));
@@ -1064,7 +1178,8 @@ int fsmc_plan_launch(fsmc_ctx* ctx, fsmc_plan* plan)
       fc.fn<<<plan->blocks, plan->threads, plan->smemBytes, st>>>(fm, a);
       if (plan->sumOnFast) {
         fsmc::sumScratchReduceKernel<<<ctx->prop.multiProcessorCount * 8, 256, 0, st>>>(ctx->sumScratch.p, sumWarps, sumPlanes, m.L,
-                                                                                        ctx->model.S, m.Spad, plan->sumPosterior.p);
+                                                                                        ctx->model.S, m.Spad, a.sumPosterior,
+                                                                                        a.stateWeight);
         plan->launches += 1;
       }
       if (plan->sparse) {
@@ -1096,6 +1211,11 @@ int fsmc_plan_launch(fsmc_ctx* ctx, fsmc_plan* plan)
   plan->launched = true;
   return FSMC_OK;
 }
+
+namespace
+{
+void fillStats(fsmc_ctx* ctx, const fsmc_plan* plan, long long found, int64_t d2h, fsmc_decode_stats* stats);
+}  // namespace
 
 int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request* out, fsmc_decode_stats* stats)
 {
@@ -1132,6 +1252,7 @@ int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request*
   const long long found = static_cast<long long>(counters[0]);
   const long long stored = std::min<long long>(found, plan->segmentCapacity);
   int rc = FSMC_OK;
+  int64_t d2h = 0;
   if (flags & FSMC_CALL_SEGMENTS) {
     if (stored > 0) {
       if (!out->segments || out->segmentCapacity < stored) {
@@ -1143,6 +1264,7 @@ int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request*
       FSMC_CUDA(ctx->segmentSorter.sort(plan->segments.p, stored, static_cast<uint32_t>(plan->numTiles * 32), st, &sorted));
       FSMC_CUDA(ctx->segStage.ensure(static_cast<size_t>(stored)));
       FSMC_CUDA(cudaMemcpyAsync(ctx->segStage.p, sorted, stored * sizeof(fsmc_segment), cudaMemcpyDeviceToHost, st));
+      d2h += stored * static_cast<int64_t>(sizeof(fsmc_segment));
     }
   }
   const size_t nSite = static_cast<size_t>(plan->numTiles) * 32 * static_cast<size_t>(plan->siteStride);
@@ -1151,18 +1273,21 @@ int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request*
       return fail(FSMC_E_INVALID, "fsmc_plan_collect: siteMean is NULL");
     }
     FSMC_CUDA(cudaMemcpyAsync(out->siteMean, plan->siteMean.p, nSite * sizeof(float), cudaMemcpyDeviceToHost, st));
+    d2h += nSite * sizeof(float);
   }
   if ((flags & FSMC_SITE_MAP) && nSite) {
     if (!out->siteMap) {
       return fail(FSMC_E_INVALID, "fsmc_plan_collect: siteMap is NULL");
     }
     FSMC_CUDA(cudaMemcpyAsync(out->siteMap, plan->siteMap.p, nSite * sizeof(int), cudaMemcpyDeviceToHost, st));
+    d2h += nSite * sizeof(int);
   }
   if ((flags & FSMC_SITE_IBD) && nSite) {
     if (!out->siteIbd) {
       return fail(FSMC_E_INVALID, "fsmc_plan_collect: siteIbd is NULL");
     }
     FSMC_CUDA(cudaMemcpyAsync(out->siteIbd, plan->siteIbd.p, nSite * sizeof(float), cudaMemcpyDeviceToHost, st));
+    d2h += nSite * sizeof(float);
   }
   if ((flags & FSMC_SITE_POSTERIOR) && nSite) {
     if (!out->sitePosterior) {
@@ -1170,6 +1295,7 @@ int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request*
     }
     FSMC_CUDA(cudaMemcpyAsync(out->sitePosterior, plan->sitePosterior.p,
                               nSite * static_cast<size_t>(ctx->model.S) * sizeof(float), cudaMemcpyDeviceToHost, st));
+    d2h += nSite * static_cast<size_t>(ctx->model.S) * sizeof(float);
   }
   if (flags & FSMC_SUM_POSTERIOR) {
     if (!out->sumPosterior) {
@@ -1177,6 +1303,7 @@ int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request*
     }
     FSMC_CUDA(cudaMemcpyAsync(out->sumPosterior, plan->sumPosterior.p, sumPosteriorCount(ctx->model, flags) * sizeof(float),
                               cudaMemcpyDeviceToHost, st));
+    d2h += sumPosteriorCount(ctx->model, flags) * sizeof(float);
   }
   FSMC_CUDA(cudaEventRecord(ctx->ev[3], st));
   FSMC_CUDA(cudaStreamSynchronize(st));
@@ -1203,6 +1330,15 @@ int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request*
   if (found > plan->segmentCapacity) {
     rc = fail(FSMC_E_OVERFLOW, "fsmc_plan_collect: %lld segments found, capacity %lld", found, plan->segmentCapacity);
   }
+  fillStats(ctx, plan, found, d2h, stats);
+  plan->launched = false;
+  return rc;
+}
+
+namespace
+{
+void fillStats(fsmc_ctx* ctx, const fsmc_plan* plan, const long long found, const int64_t d2h, fsmc_decode_stats* stats)
+{
   if (stats) {
     stats->numSegments = found;
     stats->pairSites = plan->pairSites;
@@ -1222,10 +1358,10 @@ int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request*
     stats->sparseItems = plan->sparse ? plan->itemsFound : 0;
     stats->checkpointBytes = plan->sparse ? plan->ckptSlots * static_cast<int64_t>(ctx->kernelModel.Spad) * 32 * 4 : 0;
     stats->checkpointSites = plan->sparse ? (1 << plan->ckptShift) : 0;
+    stats->d2hBytes = d2h;
   }
-  plan->launched = false;
-  return rc;
 }
+}  // namespace
 
 int fsmc_plan_destroy(fsmc_ctx* ctx, fsmc_plan* plan)
 {
@@ -1666,6 +1802,95 @@ int fsmc_decode(fsmc_ctx* ctx, const fsmc_decode_request* req, fsmc_decode_stats
                  ms(t3, std::chrono::steady_clock::now()));
   }
   return rc;
+}
+
+int fsmc_decode_device(fsmc_ctx* ctx, const fsmc_decode_request* req, const fsmc_device_outputs* out, fsmc_decode_stats* stats)
+{
+  if (!ctx || !req || !out) {
+    return fail(FSMC_E_INVALID, "fsmc_decode_device: NULL argument");
+  }
+  FSMC_CUDA(cudaSetDevice(ctx->device));
+  FSMC_CUDA(cudaEventRecord(ctx->ev[0], ctx->stream));
+  fsmc_plan* plan = nullptr;
+  int rc = planCreate(ctx, req, out, &plan);
+  if (rc != FSMC_OK) {
+    return rc;
+  }
+  rc = fsmc_plan_launch(ctx, plan);
+  if (rc == FSMC_OK) {
+    const cudaError_t e = cudaEventRecord(ctx->ev[3], ctx->stream);
+    const cudaError_t e2 = e == cudaSuccess ? cudaStreamSynchronize(ctx->stream) : e;
+    if (e2 != cudaSuccess) {
+      rc = fail(FSMC_E_CUDA, "fsmc_decode_device: %s", cudaGetErrorString(e2));
+    } else {
+      fillStats(ctx, plan, 0, 0, stats);
+    }
+  }
+  plan->launched = false;
+  const std::string keep = gLastError;
+  fsmc_plan_destroy(ctx, plan);
+  gLastError = keep;
+  return rc;
+}
+
+}  // extern "C"
+
+namespace
+{
+template <class T>
+int columnMin(fsmc_ctx* ctx, const char* name, const T* m, const int64_t rows, const int64_t cols, const int64_t ld, T* minOut,
+              int32_t* argOut)
+{
+  if (!ctx || !m || !minOut || !argOut) {
+    return fail(FSMC_E_INVALID, "%s: NULL argument", name);
+  }
+  if (rows < 1 || rows > 0x7fffffffll || cols < 1 || ld < cols) {
+    return fail(FSMC_E_INVALID, "%s: rows=%lld cols=%lld ld=%lld (need 1 <= rows < 2^31, 1 <= cols <= ld)", name,
+                static_cast<long long>(rows), static_cast<long long>(cols), static_cast<long long>(ld));
+  }
+  for (const auto& [p, what] : {std::make_pair(static_cast<const void*>(m), "m_dev"), std::make_pair(static_cast<const void*>(minOut), "min_dev"),
+                                std::make_pair(static_cast<const void*>(argOut), "argmin_dev")}) {
+    const int rc = checkDevicePtr(ctx, p, what);
+    if (rc != FSMC_OK) {
+      return rc;
+    }
+  }
+  FSMC_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  // rows are cut into chunks until the grid has about 16 blocks of 256 threads per SM
+  const long long colBlocks = (cols + fsmc::kColMinCols - 1) / fsmc::kColMinCols;
+  const long long want = (16ll * ctx->prop.multiProcessorCount + colBlocks - 1) / colBlocks;
+  const long long chunks = std::max(1ll, std::min<long long>({want, static_cast<long long>((rows + 255) / 256), 65535ll}));
+  const long long rowsPerChunk = (rows + chunks - 1) / chunks;
+  const dim3 block(fsmc::kColMinCols, fsmc::kColMinGroups);
+  const dim3 grid(static_cast<unsigned>(colBlocks), static_cast<unsigned>(chunks));
+  if (chunks == 1) {
+    fsmc::columnMinPartialKernel<T><<<grid, block, 0, st>>>(m, rows, cols, ld, rowsPerChunk, minOut, argOut);
+  } else {
+    FSMC_CUDA(ctx->colMinPart.ensure(2 * static_cast<size_t>(chunks) * cols));
+    T* partV = reinterpret_cast<T*>(ctx->colMinPart.p);
+    int* partRow = reinterpret_cast<int*>(ctx->colMinPart.p + static_cast<size_t>(chunks) * cols);
+    fsmc::columnMinPartialKernel<T><<<grid, block, 0, st>>>(m, rows, cols, ld, rowsPerChunk, partV, partRow);
+    const int cb = static_cast<int>(std::min<long long>((cols + 255) / 256, 8ll * ctx->prop.multiProcessorCount));
+    fsmc::columnMinCombineKernel<T><<<cb, 256, 0, st>>>(partV, partRow, static_cast<int>(chunks), cols, minOut, argOut);
+  }
+  FSMC_CUDA(cudaGetLastError());
+  return FSMC_OK;
+}
+}  // namespace
+
+extern "C" {
+
+int fsmc_column_min_f32(fsmc_ctx* ctx, const float* m_dev, const int64_t rows, const int64_t cols, const int64_t ld, float* min_dev,
+                        int32_t* argmin_dev)
+{
+  return columnMin(ctx, "fsmc_column_min_f32", m_dev, rows, cols, ld, min_dev, argmin_dev);
+}
+
+int fsmc_column_min_i32(fsmc_ctx* ctx, const int32_t* m_dev, const int64_t rows, const int64_t cols, const int64_t ld,
+                        int32_t* min_dev, int32_t* argmin_dev)
+{
+  return columnMin(ctx, "fsmc_column_min_i32", m_dev, rows, cols, ld, min_dev, argmin_dev);
 }
 
 }  // extern "C"

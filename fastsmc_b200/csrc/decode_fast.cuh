@@ -1040,6 +1040,7 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeFastKernel(const Fa
     const bool laneActive = lane < nPairs;
     const int srcLane = laneActive ? lane : nPairs - 1;
     const uint32_t pair = static_cast<uint32_t>(tile) * 32u + static_cast<uint32_t>(lane);
+    const uint32_t outRow = args.laneRow ? __ldg(args.laneRow + pair) : pair;  // output row (fsmc_decode_device)
     PairBits bits;
     bits.a = m.haps + static_cast<size_t>(args.hapA[static_cast<size_t>(tile) * 32 + srcLane]) * m.wordsPerHap;
     bits.b = m.haps + static_cast<size_t>(args.hapB[static_cast<size_t>(tile) * 32 + srcLane]) * m.wordsPerHap;
@@ -1180,10 +1181,10 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeFastKernel(const Fa
           }
           if (laneActive) {
             if (flags & FSMC_SITE_MEAN) {
-              args.siteMean[static_cast<size_t>(pair) * args.siteStride + p] = mean * r;
+              args.siteMean[static_cast<size_t>(outRow) * args.siteStride + p] = mean * r;
             }
             if (flags & FSMC_SITE_MAP) {
-              args.siteMap[static_cast<size_t>(pair) * args.siteStride + p] = arg;
+              args.siteMap[static_cast<size_t>(outRow) * args.siteStride + p] = arg;
             }
           }
         }
@@ -1235,7 +1236,7 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeFastKernel(const Fa
           forStatesBelow<S_T>(sT, [&](const int k) { ibdRaw += w[k]; });
           const float ibd = ibdRaw * r;
           if ((flags & FSMC_SITE_IBD) && laneActive) {
-            args.siteIbd[static_cast<size_t>(pair) * args.siteStride + p] = ibd;
+            args.siteIbd[static_cast<size_t>(outRow) * args.siteStride + p] = ibd;
           }
           if (inScan) {
             int now = -1;
@@ -1357,9 +1358,11 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeFastKernel(const Fa
   }
 }
 
-// out[(plane * S + k) * L + site] = sum over warps of scratch[warp][plane][site][k], warps in ascending order
+// out[(plane * S + k) * L + site] = sum over warps of scratch[warp][plane][site][k], warps in ascending order;
+// with a weight vector (fsmc_decode_device): out[...] += sum * weight[k] instead
 static __global__ void sumScratchReduceKernel(const float* __restrict__ scratch, const int warps, const int planes, const int L,
-                                              const int S, const int Spad, float* __restrict__ out)
+                                              const int S, const int Spad, float* __restrict__ out,
+                                              const float* __restrict__ weight = nullptr)
 {
   const long long total = static_cast<long long>(planes) * L * Spad;
   for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
@@ -1374,7 +1377,8 @@ static __global__ void sumScratchReduceKernel(const float* __restrict__ scratch,
     for (int w = 0; w < warps; ++w) {
       sum += scratch[static_cast<size_t>(w) * total + i];
     }
-    out[(plane * S + k) * L + site] = sum;
+    float* o = out + (plane * S + k) * L + site;
+    *o = weight ? __fadd_rn(*o, __fmul_rn(sum, weight[k])) : sum;
   }
 }
 

@@ -96,6 +96,9 @@ struct DecodeArgs {
   unsigned long long* refineCounter;
   // ---- sums of posteriors over pairs on the production kernel: private accumulators per resident warp ------------------
   float* sumScratch;                // [warp][planes][L][Spad]
+  // ---- fsmc_decode_device: caller-owned outputs --------------------------------------------------------------------
+  const uint32_t* laneRow;          // [numTiles*32] output row of pair tile*32+lane; NULL = the pair number
+  const float* stateWeight;         // [S] posterior rows are multiplied by it; sums are added to the output times it
 };
 
 // ---- arithmetic: EXACT = separate IEEE multiply and add (never contracted), else FMA ------------
@@ -351,7 +354,7 @@ struct CallerState {
 template <int S_T, bool EXACT, class VecA, class VecC>
 __device__ __forceinline__ void sweepForward(const DeviceModel& m, const DecodeArgs& args, PairBits& bits,
                                              const int from, const int len, const int scanFrom, const int scanTo,
-                                             const uint32_t pair, const bool laneActive, VecA& a, VecC& c,
+                                             const uint32_t pair, const uint32_t outRow, const bool laneActive, VecA& a, VecC& c,
                                              const float* __restrict__ beta, float* acc /* smem + lane */)
 {
   const int S = S_T ? S_T : m.S;
@@ -469,25 +472,27 @@ __device__ __forceinline__ void sweepForward(const DeviceModel& m, const DecodeA
       }
       if (laneActive) {
         if (flags & FSMC_SITE_MEAN) {
-          args.siteMean[static_cast<size_t>(pair) * args.siteStride + p] = mean;
+          args.siteMean[static_cast<size_t>(outRow) * args.siteStride + p] = mean;
         }
         if (flags & FSMC_SITE_MAP) {
-          args.siteMap[static_cast<size_t>(pair) * args.siteStride + p] = arg;
+          args.siteMap[static_cast<size_t>(outRow) * args.siteStride + p] = arg;
         }
       }
     }
 
     // ---- full posteriors and their sum over pairs (ref HMM.cpp:1372-1389, 1044-1085) ----------
     if (flags & (FSMC_SITE_POSTERIOR | FSMC_SUM_POSTERIOR)) {
-      float* postRow = args.sitePosterior + static_cast<size_t>(pair) * S * args.siteStride + p;
+      float* postRow = args.sitePosterior + static_cast<size_t>(outRow) * S * args.siteStride + p;
       // plane of the sum this lane's pair contributes to: its genotype class at the site, or the only plane
       const int plane = (flags & FSMC_SUM_BY_GENOTYPE) ? bits.cls(site) : 0;
       const int nPlanes = (flags & FSMC_SUM_BY_GENOTYPE) ? 3 : 1;
 #pragma unroll
       for (int k = 0; k < S; ++k) {
         const float post = __fmul_rn(c.get(k), r);
+        // fsmc_decode_device: weighted rows and sums (the host's posterior * expectedTimes[k], one rounding)
+        const float w = args.stateWeight ? __ldg(args.stateWeight + k) : 1.f;
         if ((flags & FSMC_SITE_POSTERIOR) && laneActive) {
-          postRow[static_cast<size_t>(k) * args.siteStride] = post;
+          postRow[static_cast<size_t>(k) * args.siteStride] = args.stateWeight ? __fmul_rn(post, w) : post;
         }
         if (flags & FSMC_SUM_POSTERIOR) {
           for (int pl = 0; pl < nPlanes; ++pl) {
@@ -497,7 +502,7 @@ __device__ __forceinline__ void sweepForward(const DeviceModel& m, const DecodeA
               v += __shfl_xor_sync(kFull, v, d);
             }
             if (lane0 && v != 0.f) {
-              atomicAdd(args.sumPosterior + (static_cast<size_t>(pl) * S + k) * m.L + site, v);
+              atomicAdd(args.sumPosterior + (static_cast<size_t>(pl) * S + k) * m.L + site, args.stateWeight ? __fmul_rn(v, w) : v);
             }
           }
         }
@@ -510,7 +515,7 @@ __device__ __forceinline__ void sweepForward(const DeviceModel& m, const DecodeA
       float ibd = 0.f;
       forStatesBelow<S_T>(sT, [&](const int k) { ibd = __fadd_rn(ibd, __fmul_rn(c.get(k), r)); });
       if ((flags & FSMC_SITE_IBD) && laneActive) {
-        args.siteIbd[static_cast<size_t>(pair) * args.siteStride + p] = ibd;
+        args.siteIbd[static_cast<size_t>(outRow) * args.siteStride + p] = ibd;
       }
 
       if (inScan) {
@@ -604,6 +609,7 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeTilesKernel(const D
     const bool laneActive = lane < nPairs;
     const int srcLane = laneActive ? lane : nPairs - 1;  // padding repeats the last pair (ref HMM.cpp:616-619)
     const uint32_t pair = static_cast<uint32_t>(tile) * 32u + static_cast<uint32_t>(lane);
+    const uint32_t outRow = args.laneRow ? __ldg(args.laneRow + pair) : pair;  // output row (fsmc_decode_device)
     PairBits bits;
     bits.a = m.haps + static_cast<size_t>(args.hapA[static_cast<size_t>(tile) * 32 + srcLane]) * m.wordsPerHap;
     bits.b = m.haps + static_cast<size_t>(args.hapB[static_cast<size_t>(tile) * 32 + srcLane]) * m.wordsPerHap;
@@ -611,17 +617,17 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeTilesKernel(const D
     if constexpr (MODE == 0) {
       RegVec<S_T> v0, v1;
       sweepBackward<S_T, EXACT>(m, bits, from, len, v0, v1, beta);
-      sweepForward<S_T, EXACT>(m, args, bits, from, len, scanFrom, scanTo, pair, laneActive, v0, v1, beta, acc);
+      sweepForward<S_T, EXACT>(m, args, bits, from, len, scanFrom, scanTo, pair, outRow, laneActive, v0, v1, beta, acc);
     } else if constexpr (MODE == 1) {
       RegVec<S_T> v0;
       SmemVec v1{mine + static_cast<size_t>(accRows) * 32};
       sweepBackward<S_T, EXACT>(m, bits, from, len, v0, v1, beta);
-      sweepForward<S_T, EXACT>(m, args, bits, from, len, scanFrom, scanTo, pair, laneActive, v0, v1, beta, acc);
+      sweepForward<S_T, EXACT>(m, args, bits, from, len, scanFrom, scanTo, pair, outRow, laneActive, v0, v1, beta, acc);
     } else {
       SmemVec v1{mine + static_cast<size_t>(accRows) * 32};
       SmemVec v0{mine + static_cast<size_t>(accRows + S) * 32};
       sweepBackward<0, EXACT>(m, bits, from, len, v0, v1, beta);
-      sweepForward<0, EXACT>(m, args, bits, from, len, scanFrom, scanTo, pair, laneActive, v0, v1, beta, acc);
+      sweepForward<0, EXACT>(m, args, bits, from, len, scanFrom, scanTo, pair, outRow, laneActive, v0, v1, beta, acc);
     }
     __syncwarp();
   }

@@ -710,6 +710,7 @@ __global__ void __launch_bounds__(kLaneQuarters * 32, MIN_BLOCKS) decodeLaneWide
     const bool laneActive = pairInTile < nPairs;
     const int srcPair = laneActive ? pairInTile : nPairs - 1;
     const uint32_t pair = static_cast<uint32_t>(tile) * 32u + static_cast<uint32_t>(pairInTile);
+    const uint32_t outRow = args.laneRow ? __ldg(args.laneRow + pair) : pair;  // output row (fsmc_decode_device)
     PairBits bits;
     bits.a = m.haps + static_cast<size_t>(args.hapA[static_cast<size_t>(tile) * 32 + srcPair]) * m.wordsPerHap;
     bits.b = m.haps + static_cast<size_t>(args.hapB[static_cast<size_t>(tile) * 32 + srcPair]) * m.wordsPerHap;
@@ -852,10 +853,10 @@ __global__ void __launch_bounds__(kLaneQuarters * 32, MIN_BLOCKS) decodeLaneWide
           }
           if (g == 0 && laneActive) {
             if (flags & FSMC_SITE_MEAN) {
-              args.siteMean[static_cast<size_t>(pair) * args.siteStride + p] = mean * r;
+              args.siteMean[static_cast<size_t>(outRow) * args.siteStride + p] = mean * r;
             }
             if (flags & FSMC_SITE_MAP) {
-              args.siteMap[static_cast<size_t>(pair) * args.siteStride + p] = best > 0.f ? arg : 0;
+              args.siteMap[static_cast<size_t>(outRow) * args.siteStride + p] = best > 0.f ? arg : 0;
             }
           }
         }
@@ -864,7 +865,7 @@ __global__ void __launch_bounds__(kLaneQuarters * 32, MIN_BLOCKS) decodeLaneWide
           forStatesBelow<SEG>(sT, [&](const int k) { ibdRaw += w[k]; });  // meaningful in quarter 0 (sT <= SEG)
           const float ibd = __shfl_sync(kFull, ibdRaw, pl) * r;
           if ((flags & FSMC_SITE_IBD) && g == 0 && laneActive) {
-            args.siteIbd[static_cast<size_t>(pair) * args.siteStride + p] = ibd;
+            args.siteIbd[static_cast<size_t>(outRow) * args.siteStride + p] = ibd;
           }
           if (inScan) {
             // every lane of a pair runs the same run-length state machine on the same numbers; quarter 0 emits

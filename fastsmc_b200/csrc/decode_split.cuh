@@ -409,6 +409,8 @@ __device__ __forceinline__ void splitBody(const FastModel& fm, const DecodeArgs&
     const bool laneActive = lane < nPairs;
     const int srcLane = laneActive ? lane : nPairs - 1;
     const uint32_t pair = static_cast<uint32_t>(tile) * 32u + static_cast<uint32_t>(lane);
+    // output row (fsmc_decode_device); the narrow kernels write pair-numbered rows only
+    const uint32_t outRow = (!NARROW && args.laneRow) ? __ldg(args.laneRow + pair) : pair;
     PairBits bits;
     bits.a = m.haps + static_cast<size_t>(args.hapA[static_cast<size_t>(tile) * 32 + srcLane]) * m.wordsPerHap;
     bits.b = m.haps + static_cast<size_t>(args.hapB[static_cast<size_t>(tile) * 32 + srcLane]) * m.wordsPerHap;
@@ -866,7 +868,7 @@ __device__ __forceinline__ void splitBody(const FastModel& fm, const DecodeArgs&
           const float r = 1.0f / sumParts<NW>(xc[kXPart], lane);  // ref HMM.cpp:681-685
           if (wantSite && GID == 0 && laneActive) {
             if (flags & FSMC_SITE_MEAN) {
-              args.siteMean[static_cast<size_t>(pair) * args.siteStride + p] = sumParts<NW>(xc[kXMean], lane) * r;
+              args.siteMean[static_cast<size_t>(outRow) * args.siteStride + p] = sumParts<NW>(xc[kXMean], lane) * r;
             }
             if (flags & FSMC_SITE_MAP) {
               float best = 0.f;
@@ -879,13 +881,13 @@ __device__ __forceinline__ void splitBody(const FastModel& fm, const DecodeArgs&
                   arg = __float_as_int(xc[kXArg][g][lane]);
                 }
               }
-              args.siteMap[static_cast<size_t>(pair) * args.siteStride + p] = arg;
+              args.siteMap[static_cast<size_t>(outRow) * args.siteStride + p] = arg;
             }
           }
           if (wantIbd) {
             const float ibd = xc[kXIbd][0][lane] * r;
             if ((flags & FSMC_SITE_IBD) && GID == 0 && laneActive) {
-              args.siteIbd[static_cast<size_t>(pair) * args.siteStride + p] = ibd;
+              args.siteIbd[static_cast<size_t>(outRow) * args.siteStride + p] = ibd;
             }
             if (inScan) {
               // every warp runs the same run-length state machine on the same numbers; warp 0 emits

@@ -48,9 +48,11 @@ void ASMC::ASMC::decodePairs(const std::vector<unsigned long>& hapIndicesA, cons
   mHmm.getDecodePairsReturnStruct().finaliseCalculations();
 }
 
+namespace
+{
 // ref: ASMC.cpp:102-128 — ids of the form "<IID>#1" / "<IID>#2"
-void ASMC::ASMC::decodePairs(const std::vector<std::string>& hapIdsA, const std::vector<std::string>& hapIdsB,
-                             bool perPairPosteriors, bool sumOfPosteriors, bool perPairPosteriorMeans, bool perPairMAPs)
+std::pair<std::vector<unsigned long>, std::vector<unsigned long>> hapIndicesOfIds(const Data& data, const std::vector<std::string>& hapIdsA,
+                                                                                  const std::vector<std::string>& hapIdsB)
 {
   if (hapIdsA.size() != hapIdsB.size()) {
     throw std::runtime_error("Vector of A IDs (" + std::to_string(hapIdsA.size()) +
@@ -60,10 +62,47 @@ void ASMC::ASMC::decodePairs(const std::vector<std::string>& hapIdsA, const std:
   for (size_t i = 0; i < hapIdsA.size(); ++i) {
     const auto [idA, hapA] = asmc::combinedIdToIndPlusHap(hapIdsA[i]);
     const auto [idB, hapB] = asmc::combinedIdToIndPlusHap(hapIdsB[i]);
-    a[i] = asmc::dipToHapId(asmc::getIndIdxFromIdString(mData.IIDList, idA), hapA);
-    b[i] = asmc::dipToHapId(asmc::getIndIdxFromIdString(mData.IIDList, idB), hapB);
+    a[i] = asmc::dipToHapId(asmc::getIndIdxFromIdString(data.IIDList, idA), hapA);
+    b[i] = asmc::dipToHapId(asmc::getIndIdxFromIdString(data.IIDList, idB), hapB);
   }
+  return {a, b};
+}
+}  // namespace
+
+void ASMC::ASMC::decodePairs(const std::vector<std::string>& hapIdsA, const std::vector<std::string>& hapIdsB,
+                             bool perPairPosteriors, bool sumOfPosteriors, bool perPairPosteriorMeans, bool perPairMAPs)
+{
+  const auto [a, b] = hapIndicesOfIds(mData, hapIdsA, hapIdsB);
   decodePairs(a, b, perPairPosteriors, sumOfPosteriors, perPairPosteriorMeans, perPairMAPs);
+}
+
+ASMC::ASMC::PairIndices ASMC::ASMC::decodePairsToDevice(const std::vector<unsigned long>& hapIndicesA,
+                                                        const std::vector<unsigned long>& hapIndicesB, const HMM::DeviceOutputs& out)
+{
+  if (hapIndicesA.empty() || hapIndicesA.size() != hapIndicesB.size()) {
+    throw std::runtime_error("Vector of A indices (" + std::to_string(hapIndicesA.size()) +
+                             ") must be the same size as vector of B indices (" + std::to_string(hapIndicesB.size()) +
+                             ").\n");
+  }
+  PairIndices indices(hapIndicesA.size());
+  const unsigned long numHaps = mData.numLoadedHaplotypes();
+  for (size_t i = 0; i < hapIndicesA.size(); ++i) {
+    const unsigned long a = hapIndicesA[i], b = hapIndicesB[i];
+    if (a >= numHaps || b >= numHaps) {
+      throw std::runtime_error("haplotype index out of range");
+    }
+    indices[i] = std::make_tuple(a, asmc::indPlusHapToCombinedId(mData.IIDList.at(a / 2), 1 + a % 2), b,
+                                 asmc::indPlusHapToCombinedId(mData.IIDList.at(b / 2), 1 + b % 2));
+  }
+  mHmm.decodeHapPairsToDevice(hapIndicesA, hapIndicesB, out);
+  return indices;
+}
+
+ASMC::ASMC::PairIndices ASMC::ASMC::decodePairsToDevice(const std::vector<std::string>& hapIdsA, const std::vector<std::string>& hapIdsB,
+                                                        const HMM::DeviceOutputs& out)
+{
+  const auto [a, b] = hapIndicesOfIds(mData, hapIdsA, hapIdsB);
+  return decodePairsToDevice(a, b, out);
 }
 
 DecodePairsReturnStruct ASMC::ASMC::getCopyOfResults()

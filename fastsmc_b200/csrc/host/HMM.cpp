@@ -175,6 +175,7 @@ HMM::HMM(Data _data, const DecodingParams& _decodingParams, int /*_scalingSkip*/
   m_flushPairs = static_cast<size_t>(m_batchSize) * 8192;
   if (const char* e = std::getenv("FSMC_FLUSH_BATCHES")) {  // development: reference batches per decode call
     m_flushPairs = static_cast<size_t>(m_batchSize) * static_cast<size_t>(std::max(1, std::atoi(e)));
+    m_perSiteChunkCap = m_flushPairs;
   }
   const double tUpload = now();
   uploadModel();
@@ -488,14 +489,19 @@ void HMM::decodeHapPair(const unsigned long i, const unsigned long j)
   if (static_cast<int>(m_observationsBatch.size()) == m_batchSize) {
     m_observationsBatch.clear();  // the reference's buffer empties when a batch is decoded (ref: HMM.cpp:589)
   }
-  m_pendingRow.push_back(m_decodePairsReturnStruct.getNumWritten() + m_pending.size());
+  m_pendingRow.push_back(m_deviceOut ? m_deviceRowsQueued++ : m_decodePairsReturnStruct.getNumWritten() + m_pending.size());
   m_pending.push_back(Pending{static_cast<uint32_t>(i), static_cast<uint32_t>(j), 0u, static_cast<uint32_t>(data.sites)});
   // per-site outputs are pairs x sites floats: keep chunks small enough for host and device buffers
   // (full posterior matrices are states times larger)
   const size_t perPairFloats = std::max<size_t>(1, static_cast<size_t>(data.sites)) *
-                               (m_storePerPairPosterior ? static_cast<size_t>(m_decodingQuant.states) + 2 : 2);
-  const size_t perSiteChunk = std::max<size_t>(static_cast<size_t>(m_batchSize),
-                                               (size_t{1} << 29) / perPairFloats / m_batchSize * m_batchSize);
+                               ((m_deviceOut ? m_deviceOut->perPairPosteriors != nullptr : m_storePerPairPosterior)
+                                   ? static_cast<size_t>(m_decodingQuant.states) + 2
+                                   : 2);
+  size_t perSiteChunk = std::max<size_t>(static_cast<size_t>(m_batchSize),
+                                         (size_t{1} << 29) / perPairFloats / m_batchSize * m_batchSize);
+  if (m_perSiteChunkCap > 0) {
+    perSiteChunk = std::min(perSiteChunk, m_perSiteChunkCap);
+  }
   if (!decodingParams.FastSMC && m_pending.size() >= perSiteChunk) {
     flushPending(false);
   }
@@ -549,6 +555,8 @@ void HMM::flushPending(const bool all)
   const bool store = m_storePerPairPosteriorMean || m_storePerPairMAP || m_storePerPairPosterior || m_storeSumOfPosterior;
   if (segments) {
     runSegmentChunk(m_pending.data(), n);
+  } else if (m_deviceOut) {
+    runDeviceChunk(m_pending.data(), m_pendingRow.data(), n);
   } else {
     // ref: HMM.cpp:570-581 (addToBatch) — the sums over pairs and the per-pair outputs are independent consumers of the
     // same batch: both run when both are asked for
@@ -958,6 +966,7 @@ void HMM::runPerSiteChunk(const Pending* pend, const unsigned long* rows, const 
   m_stats.pairSites += st.pairSites;
   m_stats.kernelMs += st.kernelMs;
   m_stats.deviceMs += st.totalMs;
+  m_stats.d2hBytes += static_cast<double>(st.d2hBytes);
   auto& out = m_decodePairsReturnStruct;
   for (size_t tile = 0; tile < T; ++tile) {
     for (int lane = 0; lane < t.pairs[tile]; ++lane) {
@@ -1000,6 +1009,73 @@ void HMM::runPerSiteChunk(const Pending* pend, const unsigned long* rows, const 
       }
     }
   }
+}
+
+void HMM::decodeHapPairsToDevice(const std::vector<unsigned long>& hapsA, const std::vector<unsigned long>& hapsB,
+                                 const DeviceOutputs& out)
+{
+  if (!m_pending.empty() || decodingParams.FastSMC) {
+    throw std::runtime_error("HMM::decodeHapPairsToDevice: needs ASMC mode (no segment calling) and no pairs still queued");
+  }
+  check(fsmc_ctx_set_stream(m_ctx, out.stream), "fsmc_ctx_set_stream");
+  m_deviceOut = &out;
+  m_deviceRowsQueued = 0;
+  try {
+    decodeHapPairs(hapsA, hapsB);
+    finishDecoding();
+  } catch (...) {
+    m_pending.clear();
+    m_pendingRow.clear();
+    m_deviceOut = nullptr;
+    fsmc_ctx_set_stream(m_ctx, nullptr);
+    throw;
+  }
+  m_deviceOut = nullptr;
+  check(fsmc_ctx_set_stream(m_ctx, nullptr), "fsmc_ctx_set_stream");
+}
+
+// The outputs of runPerSiteChunk, written by the kernels into the caller's device rows (fsmc_decode_device)
+void HMM::runDeviceChunk(const Pending* pend, const unsigned long* rows, const size_t n)
+{
+  const TileSet t = buildTiles(pend, n, static_cast<size_t>(m_batchSize), false, data.geneticPositions, data.sites);
+  const size_t T = t.pairs.size();
+  const DeviceOutputs& o = *m_deviceOut;
+  fsmc_decode_request req{};
+  req.numTiles = static_cast<int64_t>(T);
+  req.hapA = t.hapA.data();
+  req.hapB = t.hapB.data();
+  req.tilePairs = t.pairs.data();
+  req.tileFrom = t.from.data();
+  req.tileTo = t.to.data();
+  req.flags = (o.perPairPosteriorMeans ? FSMC_SITE_MEAN : 0u) | (o.perPairMAPs ? FSMC_SITE_MAP : 0u) |
+              (o.perPairPosteriors ? FSMC_SITE_POSTERIOR : 0u) | (o.sumOfPosteriors ? FSMC_SUM_POSTERIOR : 0u) |
+              (decodingParams.exactArithmetic ? FSMC_EXACT : 0u);
+  std::vector<int64_t> laneRow(T * FSMC_TILE, 0);
+  for (size_t tile = 0; tile < T; ++tile) {
+    for (int lane = 0; lane < t.pairs[tile]; ++lane) {
+      laneRow[tile * FSMC_TILE + lane] = static_cast<int64_t>(rows[t.firstPair[tile] + lane]);
+    }
+  }
+  fsmc_device_outputs dev{};
+  dev.laneRow = laneRow.data();
+  dev.numRows = static_cast<int64_t>(m_deviceRowsQueued);
+  dev.siteStride = data.sites;
+  dev.siteMean_dev = o.perPairPosteriorMeans;
+  dev.siteMap_dev = o.perPairMAPs;
+  dev.sitePosterior_dev = o.perPairPosteriors;
+  dev.sumPosterior_dev = o.sumOfPosteriors;
+  // the reference stores posterior * expectedCoalTimes[k] (ref: HMM.cpp:1382-1389)
+  dev.stateWeight = m_decodingQuant.expectedTimes.data();
+  fsmc_decode_stats st{};
+  const double t0 = now();
+  check(fsmc_decode_device(m_ctx, &req, &dev, &st), "fsmc_decode_device");
+  m_stats.decodeWallS += now() - t0;
+  m_stats.decodeCalls += 1;
+  m_stats.pairsDecoded += n;
+  m_stats.pairSites += st.pairSites;
+  m_stats.kernelMs += st.kernelMs;
+  m_stats.deviceMs += st.totalMs;
+  m_stats.d2hBytes += static_cast<double>(st.d2hBytes);
 }
 
 // Posterior sums over all pairs of the job for ASMC's decodeAll (ref: HMM.cpp:1044-1085, augmentSumOverPairs): the

@@ -113,6 +113,21 @@ public:
   void setStorePerPairPosterior(bool v = true) { m_storePerPairPosterior = v; }
   void setStoreSumOfPosterior(bool v = true) { m_storeSumOfPosterior = v; }
 
+  /// Caller-owned device memory (of the decoding device) for decodeHapPairsToDevice; NULL = not computed.  Row r is the
+  /// r-th pair of the call.  The values are those ASMC::decodePairs stores (posteriors times expectedTimes).
+  struct DeviceOutputs {
+    float* perPairPosteriors = nullptr;      // [pairs][states][sites]
+    float* sumOfPosteriors = nullptr;        // [states][sites], added to
+    float* perPairPosteriorMeans = nullptr;  // [pairs][sites]
+    int32_t* perPairMAPs = nullptr;          // [pairs][sites]
+    void* stream = nullptr;                  // cudaStream_t the work is enqueued on (NULL: the context's own stream)
+  };
+  /// The per-pair outputs of decodeHapPairs written by the kernels straight into `out`, chunk by chunk (the chunks of the
+  /// host path, so the sums are added up in the same order).  Neither the return structure nor the posterior sums of
+  /// decodeAll (DecodingReturnValues) are touched.
+  void decodeHapPairsToDevice(const std::vector<unsigned long>& hapsA, const std::vector<unsigned long>& hapsB,
+                              const DeviceOutputs& out);
+
   // ---- B200 build: model tables as handed to fsmc_set_model, and run statistics ---------------------------------
   struct ModelTables {
     int states = 0, sites = 0, numDistances = 0;
@@ -136,9 +151,11 @@ public:
     double outputWallS = 0.0; // host wall time formatting + compressing records
     double tablesWallS = 0.0; // constructor: decoding quantities + emission / transition tables on the host
     double uploadWallS = 0.0; // constructor: context creation, model and haplotype upload
+    double d2hBytes = 0.0;    // decode outputs copied device -> host
   };
   const RunStats& getRunStats() const { return m_stats; }
   fsmc_ctx* context() { return m_ctx; }
+  int getDevice() const { return decodingParams.device; }  // CUDA device of the decode context
   /// segments of the run are also kept in memory when this is set (tests, Python callers)
   void setKeepSegments(bool keep) { m_keepSegments = keep; }
   const std::vector<IbdSegment>& getSegments() const { return m_segments; }
@@ -171,6 +188,9 @@ private:
   std::vector<Pending> m_pending;
   std::vector<unsigned long> m_pendingRow;  // row of the return struct for each pending pair (decodePairs path)
   size_t m_flushPairs = 0;
+  size_t m_perSiteChunkCap = 0;  // FSMC_FLUSH_BATCHES: also caps the per-site chunks of decodeHapPairs (0 = no cap)
+  const DeviceOutputs* m_deviceOut = nullptr;  // set during decodeHapPairsToDevice
+  unsigned long m_deviceRowsQueued = 0;        // pairs of that call queued so far
   bool m_windowed = false;  // pending pairs carry their own [from,to] (hashing) instead of [0, sites)
 
   DecodingReturnValues m_decodingReturnValues;
@@ -196,6 +216,7 @@ private:
   void runSegmentChunk(const Pending* pairs, size_t n);
   void runPerSiteChunk(const Pending* pairs, const unsigned long* rows, size_t n);
   void runPosteriorSumChunk(const Pending* pairs, size_t n);
+  void runDeviceChunk(const Pending* pairs, const unsigned long* rows, size_t n);
   IbdSegment toIbdSegment(const SegmentBlock& block, size_t i) const;
   void formatSegments(const SegmentBlock& block, size_t lo, size_t hi, std::string& out) const;
   std::atomic<double> m_segmentsPerPair{4.0};  // densest chunk so far: sizes the next chunk's record buffer

@@ -299,7 +299,8 @@ PYBIND11_MODULE(pyASMC, m)
       .def_readonly("kernelMs", &HMM::RunStats::kernelMs)
       .def_readonly("deviceMs", &HMM::RunStats::deviceMs)
       .def_readonly("decodeWallS", &HMM::RunStats::decodeWallS)
-      .def_readonly("outputWallS", &HMM::RunStats::outputWallS);
+      .def_readonly("outputWallS", &HMM::RunStats::outputWallS)
+      .def_readonly("d2hBytes", &HMM::RunStats::d2hBytes);
 
   py::class_<HMM>(m, "HMM")
       .def(py::init([](const Data& d, const DecodingParams& p, int skip) { return new HMM(d, p, skip); }), "data"_a,
@@ -321,6 +322,7 @@ PYBIND11_MODULE(pyASMC, m)
       .def("makePairObs", &HMM::makePairObs, "iHap"_a, "ind1"_a, "jHap"_a, "ind2"_a, "materialise"_a = true)
       .def("getRunStats", &HMM::getRunStats, py::return_value_policy::reference_internal)
       .def("getNumberOfDetectedSegments", &HMM::getNumberOfDetectedSegments)
+      .def("getDevice", &HMM::getDevice)
       .def("getModelTables", [](const HMM& h) { return tablesToDict(h.getModelTables(), h.getDecodingQuantities()); });
 
 
@@ -384,6 +386,30 @@ PYBIND11_MODULE(pyASMC, m)
                &ASMC::ASMC::decodePairs),
            "hap_ids_a"_a, "hap_ids_b"_a, "per_pair_posteriors"_a = false, "sum_of_posteriors"_a = false,
            "per_pair_posterior_means"_a = false, "per_pair_MAPs"_a = false)
+      // device-resident outputs: raw device pointers (e.g. torch's data_ptr()) and a cudaStream_t as integers, 0 = none;
+      // returns per_pair_indices.  fastsmc_b200.cuda_results.decode_pairs_cuda allocates and checks the tensors.
+      .def("decodePairsToDevice",
+           [](ASMC::ASMC& self, const py::object& a, const py::object& b, const uintptr_t perPairPosteriors,
+              const uintptr_t sumOfPosteriors, const uintptr_t perPairPosteriorMeans, const uintptr_t perPairMAPs,
+              const uintptr_t stream) {
+             HMM::DeviceOutputs out;
+             out.perPairPosteriors = reinterpret_cast<float*>(perPairPosteriors);
+             out.sumOfPosteriors = reinterpret_cast<float*>(sumOfPosteriors);
+             out.perPairPosteriorMeans = reinterpret_cast<float*>(perPairPosteriorMeans);
+             out.perPairMAPs = reinterpret_cast<int32_t*>(perPairMAPs);
+             out.stream = reinterpret_cast<void*>(stream);
+             const py::list la(a), lb(b);
+             if (la.size() > 0 && py::isinstance<py::str>(la[0])) {
+               const auto ia = la.cast<std::vector<std::string>>(), ib = lb.cast<std::vector<std::string>>();
+               py::gil_scoped_release release;
+               return self.decodePairsToDevice(ia, ib, out);
+             }
+             const auto ia = la.cast<std::vector<unsigned long>>(), ib = lb.cast<std::vector<unsigned long>>();
+             py::gil_scoped_release release;
+             return self.decodePairsToDevice(ia, ib, out);
+           },
+           "haps_a"_a, "haps_b"_a, "per_pair_posteriors"_a = 0, "sum_of_posteriors"_a = 0, "per_pair_posterior_means"_a = 0,
+           "per_pair_MAPs"_a = 0, "stream"_a = 0)
       .def("get_copy_of_results", &ASMC::ASMC::getCopyOfResults, py::return_value_policy::copy)
       .def("get_ref_of_results", &ASMC::ASMC::getRefOfResults, py::return_value_policy::reference_internal)
       .def("hmm", &ASMC::ASMC::hmm, py::return_value_policy::reference_internal);

@@ -175,9 +175,45 @@ typedef struct fsmc_decode_stats {
   int32_t checkpointSites;  /* sites per checkpoint block                                           */
   int64_t sparseItems;      /* run pieces (one per run and block) refined                           */
   int64_t checkpointBytes;  /* beta checkpoints in HBM                                              */
+  /* outputs copied device -> host by the call: segment records, per-site rows and sums (the counter read-back of at most
+   * 32 bytes that sizes them is not counted).  0 for fsmc_decode_device.                                              */
+  int64_t d2hBytes;
 } fsmc_decode_stats;
 
 int fsmc_decode(fsmc_ctx* ctx, const fsmc_decode_request* req, fsmc_decode_stats* stats);
+
+/* ------------------------------------------------------------------------------------------------
+ * Device-resident outputs: the per-site outputs of fsmc_decode written by the decode kernels straight into caller-owned
+ * device memory of the context's device (e.g. torch tensors), at caller-chosen rows.  Nothing is staged and nothing but
+ * the stats crosses to the host.  The request's own output fields are ignored; FSMC_CALL_SEGMENTS is rejected.  The kernel
+ * is the one fsmc_decode chooses for the same flags; a request that would run a narrow kernel (FSMC_SITE_IBD without
+ * FSMC_SITE_MEAN / FSMC_SITE_MAP) is rejected, since those kernels write pair-numbered rows only: add FSMC_WIDE_KERNEL.
+ * All work is enqueued on the context's stream; the call returns when it has completed.
+ * ------------------------------------------------------------------------------------------------ */
+typedef struct fsmc_device_outputs {
+  const int64_t* laneRow;     /* host [numTiles*32]: output row of pair tile*32+lane; ignored for unused lanes          */
+  int64_t numRows;            /* rows of every per-pair output below (< 2^31)                                         */
+  int64_t siteStride;         /* >= longest window; column = pos - tileFrom                                           */
+  float* siteMean_dev;        /* [numRows][siteStride] or NULL (FSMC_SITE_MEAN)                                       */
+  int32_t* siteMap_dev;       /* [numRows][siteStride] or NULL (FSMC_SITE_MAP)                                        */
+  float* siteIbd_dev;         /* [numRows][siteStride] or NULL (FSMC_SITE_IBD)                                        */
+  float* sitePosterior_dev;   /* [numRows][states][siteStride] or NULL (FSMC_SITE_POSTERIOR): posterior * stateWeight[k] */
+  /* [planes][states][sites] or NULL (FSMC_SUM_POSTERIOR): ACCUMULATED, out += (sum over the call's pairs) * stateWeight[k]
+   * (one rounding per operation, in this order: the host's per-chunk update of ASMC::decodePairs)                          */
+  float* sumPosterior_dev;
+  const float* stateWeight;   /* host [states] or NULL (= 1): ASMC passes expectedTimes (ref: HMM.cpp:1382-1389)       */
+} fsmc_device_outputs;
+int fsmc_decode_device(fsmc_ctx* ctx, const fsmc_decode_request* req, const fsmc_device_outputs* out,
+                       fsmc_decode_stats* stats);
+
+/* Per column of a row-major device matrix m[rows][ld] (cols <= ld): the minimum over rows and the first row that attains it,
+ * as DecodePairsReturnStruct::finaliseCalculations (ref: DecodePairsReturnStruct.hpp:105-118): row 0 is the start value and
+ * a later row replaces it only when strictly smaller (so a NaN in row 0 stays, later NaNs are skipped).  Deterministic.
+ * Enqueued on the context's stream; returns without waiting.  min_dev / argmin_dev: [cols], device memory.              */
+int fsmc_column_min_f32(fsmc_ctx* ctx, const float* m_dev, int64_t rows, int64_t cols, int64_t ld, float* min_dev,
+                        int32_t* argmin_dev);
+int fsmc_column_min_i32(fsmc_ctx* ctx, const int32_t* m_dev, int64_t rows, int64_t cols, int64_t ld, int32_t* min_dev,
+                        int32_t* argmin_dev);
 
 /* Which kernel family a request with these flags would run on the context's model, before any request exists: callers
  * that run several contexts on one device (HMM's pipelined decode workers) must know whether the request sizes its
