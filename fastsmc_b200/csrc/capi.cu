@@ -24,7 +24,7 @@
 #include "seed_order.h"
 #include "host/SeedMapOrder.hpp"
 #include "segment_sort.h"
-#include "split_select.h"
+#include "lane_select.h"
 
 namespace
 {
@@ -271,22 +271,14 @@ struct FastChoice {
   FastKernelFn fn = nullptr;
   int Spad = 0;
   int threads = 0;
-  bool acc = false;
   bool narrow = false;      // decodeNarrowKernel: sT+1 floats per pair-site in HBM instead of S
   int recordQuads = 0;
-  int splitWarps = 0;       // > 0: decodeSplitKernel, one tile per CTA of this many warps (decode_split.cuh)
-  size_t splitSmem = 0;
+  int laneWarps = 0;        // > 0: lane-split kernel, one tile per CTA of this many warps (decode_lane.cuh)
+  size_t laneSmem = 0;
   bool sparse = false;      // decodeNarrowKernel<SPARSE> + refineKernel (decode_sparse.cuh)
   bool sum = false;         // decodeFastKernel<SUM>: per-warp accumulators of the posterior sums
 };
 
-// FSMC_SPLIT=0 forces the one-warp-per-tile kernels, FSMC_SPLIT=1 the state-split kernels wherever one exists
-// (development / A-B measurements); unset = the faster of the two as measured on B200.
-int splitPreference()
-{
-  const char* e = std::getenv("FSMC_SPLIT");
-  return e && *e ? std::atoi(e) : -1;
-}
 // Without per-segment age estimates 8 warps (2 CTAs of 4) fit an SM; the accumulators of FSMC_SEG_AGE cost 8.6 KB of
 // shared memory per warp, which leaves room for 7 warps (1 CTA).
 // preferSparse: the request's scan windows are long (all-pairs decoding): IBD runs cover a small part of them
@@ -299,7 +291,7 @@ FastChoice chooseFastKernel(const DeviceModel& m, const unsigned flags, const bo
   }
   if (flags & FSMC_SUM_POSTERIOR) {
     if (S == 69 && !(flags & FSMC_CALL_SEGMENTS)) {
-      FastChoice fc{fsmc::decodeFastKernel<69, kFastDepth, kFastRescale, false, 128, 2, true>, 72, 128, false};
+      FastChoice fc{fsmc::decodeFastKernel<69, kFastDepth, kFastRescale, false, 128, 2, true>, 72, 128};
       fc.sum = true;
       return fc;
     }
@@ -310,41 +302,23 @@ FastChoice chooseFastKernel(const DeviceModel& m, const unsigned flags, const bo
   const bool narrow = !(flags & (FSMC_SITE_MEAN | FSMC_SITE_MAP | FSMC_WIDE_KERNEL)) && (!acc || m.ageThreshold <= m.stateThreshold) &&
                       m.stateThreshold + 1 <= 4 * fsmc::kNarrowMaxQuads;
   const int rqWanted = narrow ? (m.stateThreshold + 1 + 3) / 4 : 0;
-  const int pref = (flags & FSMC_ONE_WARP_KERNEL) ? 0 : splitPreference();
-  const bool trySplit = pref == 1 || (pref == -1 && S == 159);
-  if (trySplit && (S == 69 || S == 159) && m.stateThreshold <= 32) {
-    fsmc::SplitChoice sc{};
-    static const bool laneOff = [] { const char* e = std::getenv("FSMC_LANE"); return e && *e == '0'; }();  // A/B runs
-    if (S == 159 && m.laneAux && !laneOff) {
-      sc = fsmc::laneKernel159(rqWanted);  // states cut across the lanes of a warp (decode_lane.cuh)
-    }
-    if (!sc.fn) {
-      sc = S == 69 ? fsmc::splitKernel69(rqWanted, acc) : fsmc::splitKernel159(rqWanted, acc);
-    }
-    if (!sc.fn && narrow) {
-      sc = S == 69 ? fsmc::splitKernel69(0, acc) : fsmc::splitKernel159(0, acc);  // no such record width: full rows
-    }
-    if (sc.fn) {
-      FastChoice fc{sc.fn, sc.Spad, sc.warps * 32, sc.acc, sc.recordQuads > 0, sc.recordQuads};
-      fc.splitWarps = sc.warps;
-      fc.splitSmem = sc.smemBytes;
-      return fc;
-    }
+  if (S == 159 && !(flags & FSMC_ONE_WARP_KERNEL) && m.stateThreshold <= 32) {
+    const fsmc::LaneChoice lc = fsmc::laneKernel159(rqWanted);  // states cut across the lanes of a warp (decode_lane.cuh)
+    FastChoice fc{lc.fn, lc.Spad, lc.warps * 32, lc.recordQuads > 0, lc.recordQuads};
+    fc.laneWarps = lc.warps;
+    fc.laneSmem = lc.smemBytes;
+    return fc;
   }
   // all-state age estimates of sparse IBD runs: narrow sweeps + checkpoints, full posteriors only inside the runs
   const bool sparse = preferSparse && S == 69 && acc && m.ageThreshold > m.stateThreshold &&
                       !(flags & (FSMC_SITE_MEAN | FSMC_SITE_MAP | FSMC_WIDE_KERNEL)) && m.stateThreshold + 1 <= 4 * fsmc::kNarrowMaxQuads;
   if (sparse) {
     const int rq = (m.stateThreshold + 1 + 3) / 4;
-    FastKernelFn fn = rq == 1   ? fsmc::decodeNarrowKernel<69, 1, 4, kFastDepth, 128, 2, 1>
-                      : rq == 2 ? fsmc::decodeNarrowKernel<69, 2, 2, kFastDepth, 128, 2, 1>
-                      : rq == 3 ? fsmc::decodeNarrowKernel<69, 3, 2, kFastDepth, 128, 2, 1>
-                                : fsmc::decodeNarrowKernel<69, 4, 2, kFastDepth, 128, 2, 1>;
-    if (const char* e = std::getenv("FSMC_SPARSE_VARIANT")) {  // development: A/B of code-size variants
-      const int v = std::atoi(e);
-      if (rq == 1 && v == 65) fn = fsmc::decodeNarrowKernel<69, 1, 4, kFastDepth, 128, 2, 65>;  // groups fully unrolled
-    }
-    FastChoice fc{fn, 72, 128, false, true, rq};
+    FastKernelFn fn = rq == 1   ? fsmc::decodeNarrowKernel<69, 1, 4, kFastDepth, 128, 2, true>
+                      : rq == 2 ? fsmc::decodeNarrowKernel<69, 2, 2, kFastDepth, 128, 2, true>
+                      : rq == 3 ? fsmc::decodeNarrowKernel<69, 3, 2, kFastDepth, 128, 2, true>
+                                : fsmc::decodeNarrowKernel<69, 4, 2, kFastDepth, 128, 2, true>;
+    FastChoice fc{fn, 72, 128, true, rq};
     fc.sparse = true;
     return fc;
   }
@@ -356,14 +330,11 @@ FastChoice chooseFastKernel(const DeviceModel& m, const unsigned flags, const bo
                       : rq == 2 ? fsmc::decodeNarrowKernel<69, 2, 2, kFastDepth, 128, 2>
                       : rq == 3 ? fsmc::decodeNarrowKernel<69, 3, 2, kFastDepth, 128, 2>
                                 : fsmc::decodeNarrowKernel<69, 4, 2, kFastDepth, 128, 2>;
-    if (const char* e = std::getenv("FSMC_SPARSE_VARIANT")) {
-      if (rq == 1 && std::atoi(e) == 65) fn = fsmc::decodeNarrowKernel<69, 1, 4, kFastDepth, 128, 2, 64>;
-    }
-    return FastChoice{fn, 72, 128, false, true, rq};
+    return FastChoice{fn, 72, 128, true, rq};
   }
   if (S == 69) {
-    return acc ? FastChoice{fsmc::decodeFastKernel<69, kFastDepth, kFastRescale, true, 128, 2>, 72, 128, true}
-               : FastChoice{fsmc::decodeFastKernel<69, kFastDepth, kFastRescale, false, 128, 2>, 72, 128, false};
+    return acc ? FastChoice{fsmc::decodeFastKernel<69, kFastDepth, kFastRescale, true, 128, 2>, 72, 128}
+               : FastChoice{fsmc::decodeFastKernel<69, kFastDepth, kFastRescale, false, 128, 2>, 72, 128};
   }
   return {};
 }
@@ -377,8 +348,8 @@ bool sparsePreferred(const double meanScanSites)
 
 size_t fastSmemBytes(const FastChoice& fc, const int S)
 {
-  if (fc.splitWarps > 0) {
-    return fc.splitSmem;
+  if (fc.laneWarps > 0) {
+    return fc.laneSmem;
   }
   const size_t warps = fc.threads / 32;
   if (fc.narrow) {
@@ -659,7 +630,7 @@ int fsmc_query_kernel(fsmc_ctx* ctx, const uint32_t flags, const double meanScan
   out->statesKernel = fc.fn ? ctx->kernelModel.S : kc.statesKernel;
   out->narrowKernel = fc.narrow ? 1 : 0;
   out->sparseKernel = fc.sparse ? 1 : 0;
-  out->tileWarps = fc.splitWarps > 0 ? fc.splitWarps : 1;
+  out->tileWarps = fc.laneWarps > 0 ? fc.laneWarps : 1;
   out->largeScratch = (!fc.fn || !fc.narrow || fc.sparse) ? 1 : 0;
   return FSMC_OK;
 }
@@ -930,14 +901,14 @@ static int planCreate(fsmc_ctx* ctx, const fsmc_decode_request* req, const fsmc_
   plan->sparse = fc.sparse;
   plan->statesKernel = plan->fast ? ctx->kernelModel.S : kc.statesKernel;
   plan->narrow = fc.narrow;
-  plan->tileWarps = fc.splitWarps > 0 ? fc.splitWarps : 1;
+  plan->tileWarps = fc.laneWarps > 0 ? fc.laneWarps : 1;
   plan->mode = kc.mode;
   if (dev && (fc.narrow || fc.sparse)) {
     return fail(FSMC_E_INVALID, "fsmc_decode_device: flags 0x%x run a narrow kernel, which has no caller rows: set FSMC_SITE_MEAN, "
                 "FSMC_SITE_MAP or FSMC_WIDE_KERNEL", flags);
   }
-  // tiles in flight per CTA: one per warp, except for the state-split kernels (one tile per CTA)
-  int warpsPerBlock = fc.splitWarps > 0 ? 1 : (plan->fast ? fc.threads : kc.threads) / 32;
+  // tiles in flight per CTA: one per warp, except for the lane-split kernels (one tile per CTA)
+  int warpsPerBlock = fc.laneWarps > 0 ? 1 : (plan->fast ? fc.threads : kc.threads) / 32;
   const size_t smemLimit = ctx->prop.sharedMemPerBlockOptin;
   int blocksPerSm = 0;
   if (plan->fast) {

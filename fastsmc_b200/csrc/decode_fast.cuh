@@ -528,16 +528,13 @@ template <int S_T, int RQ, int G> struct NarrowSlot {
 // keeps alpha of the position before the current block in a per-warp scratch that stays in L2 and records every piece of
 // an IBD run (one item per run and block) together with that alpha.  The refine pass recomputes the full posterior only
 // inside those pieces.
-template <int S_T, int RQ, int G, int DEPTH, int THREADS, int MIN_BLOCKS, int SPARSE_V = 0>
+//
+// One copy of each step pair per sweep (`#pragma unroll 1` on the group loops): the site loops stream from the instruction
+// cache.  Fully unrolled over the group the kernel is ~100 KB of straight-line code and `no_instruction` is its first stall
+// (profiles/r2_p1_decodeNarrowSparse_packed_unrolled_ncu_full.txt: 1.61 warps per issue; 346 -> 294 ms per cfg2 step without the unrolling).
+template <int S_T, int RQ, int G, int DEPTH, int THREADS, int MIN_BLOCKS, bool SPARSE = false>
 __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const FastModel fm, const DecodeArgs args)
 {
-  constexpr bool SPARSE = (SPARSE_V & 1) != 0;
-  constexpr bool kSkipFwd = (SPARSE_V & 2) != 0, kSkipBwd = (SPARSE_V & 4) != 0;  // timing experiments only
-  // One copy of each step pair per sweep: the site loops stream from the instruction cache.  Fully unrolled over the group
-  // (bit 64, kept for A/B runs) the kernel is ~100 KB of straight-line code and `no_instruction` is its first stall
-  // (profiles/r2_p1_decodeNarrowSparse_packed_unrolled_ncu_full.txt: 1.61 warps per issue; 346 -> 294 ms per cfg2 step without the unrolling).
-  constexpr int kGroupUnroll = (SPARSE_V & 64) ? G / 2 : 1;
-  constexpr bool kSkipAlpha = (SPARSE_V & 8) != 0, kSkipBoundaryItems = (SPARSE_V & 16) != 0, kSkipRunItems = (SPARSE_V & 32) != 0;
   constexpr int S = S_T;
   constexpr int SQ = (S + 3) / 4;
   constexpr int Spad = SQ * 4;
@@ -684,7 +681,7 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const 
         const int n = min(g == 0 ? first : G, steps - j0);
         const float* coef = coefArea(slot);
         float4* stage = recArea(slot);
-        if constexpr (SPARSE && !kSkipBwd) {
+        if constexpr (SPARSE) {
           // a = beta of window position len-1-j0, the top of this group: the last position of a block?
           if (g > 0 && ((len - 1 - j0) & ckMask) == ckMask) {
             storeCheckpoint(a, len - 1 - j0);
@@ -712,7 +709,7 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const 
         };
         // The kernel is bound by instruction supply: per-SITE sparse bookkeeping made "no instruction" its first stall
         // (profiles/r2_v4_decodeNarrowSparse_ncu_full.txt), which is why that bookkeeping lives at the group tops.
-#pragma unroll(kGroupUnroll)
+#pragma unroll 1
         for (int i = 0; i < G; i += 2) {
           if (i < n) {
             step(i, a, c, false);
@@ -819,12 +816,10 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const 
           const bool closing = now >= 0 && site == scanTo - 1;
           const float rr = now >= 0 ? r : 0.f;
           const float keep = changed ? 0.f : 1.f;
-          if constexpr (SPARSE && !kSkipFwd) {
+          if constexpr (SPARSE) {
             if (__any_sync(kFull, ending || closing)) {
               // the run's last piece, then the record; the refine pass fills in the age estimates from the chain
-              if constexpr (!kSkipRunItems) {
-                emitItems(ending && runOpen && pieceStart <= site - 1, (p - 1) >> ckShift, pieceStart, site - 1);
-              }
+              emitItems(ending && runOpen && pieceStart <= site - 1, (p - 1) >> ckShift, pieceStart, site - 1);
               if (ending) {
                 emitSegment<false>(m, args, pair, cs.start, site - 1, cs.prob, cs.level, nullptr, false, chain);
                 chain = -1;
@@ -834,9 +829,7 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const 
                 runOpen = true;
                 pieceStart = site;
               }
-              if constexpr (!kSkipRunItems) {
-                emitItems(closing, p >> ckShift, pieceStart, site);
-              }
+              emitItems(closing, p >> ckShift, pieceStart, site);
               if (closing) {
                 emitSegment<false>(m, args, pair, changed ? site : cs.start, site, changed ? ibd : cs.prob + ibd, now, nullptr,
                                    false, chain);
@@ -894,20 +887,16 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const 
         float4* recs = recArea(slot);
         mbarWait(&bars[slot], (parity >> slot) & 1u);
         parity ^= 1u << slot;
-        if constexpr (SPARSE && !kSkipFwd) {
+        if constexpr (SPARSE) {
           if (g > 0 && (p0 & ckMask) == 0) {
             // a block begins with this group; c = alpha of the position before it.  A run that continues into the block
             // leaves the piece of the block that just ended (with the alpha that was parked when that block began), then
             // the new block's alpha is parked.  Same lanes write and read the scratch: no synchronisation needed.
-            if constexpr (!kSkipBoundaryItems) {
-              if (__any_sync(kFull, runOpen)) {
-                emitItems(runOpen, (p0 - 1) >> ckShift, pieceStart, from + p0 - 1);
-              }
+            if (__any_sync(kFull, runOpen)) {
+              emitItems(runOpen, (p0 - 1) >> ckShift, pieceStart, from + p0 - 1);
             }
             pieceStart = from + p0;
-            if constexpr (!kSkipAlpha) {
-              storeVector(c, alphaStart);
-            }
+            storeVector(c, alphaStart);
           }
         }
         auto step = [&](const int i, float (&x)[S], float (&y)[S], const bool rescale) {
@@ -922,7 +911,7 @@ __global__ void __launch_bounds__(THREADS, MIN_BLOCKS) decodeNarrowKernel(const 
           Z *= bPrev * sc;  // Z_p = Z_{p-1} * b_{p-1} / a_p
           consume(p, y, recs + static_cast<size_t>(i) * RQ * 32);
         };
-#pragma unroll(kGroupUnroll)
+#pragma unroll 1
         for (int i = 0; i < G; i += 2) {
           if (i == 0 && g == 0) {
             // p = 0: alpha^(0) = prior * emission into a; the one exact normaliser Z_0 = sum_k alpha^(0)[k] beta^(0)[k]

@@ -1,8 +1,8 @@
 // fastsmc_b200 — lane-split decode kernel for sm_100a (159 states, FastSMC_exe's default flags).
 //
 // At 159 states a lane cannot hold two state vectors (decode_fast.cuh), and cutting the states across the WARPS of a CTA
-// (decode_split.cuh) costs three CTA barriers per step and four different instruction streams per CTA: the profiler shows
-// `no_instruction` and `barrier` as its first two stalls (profiles/r1_v19_decodeSplit_s159_ncu_full.txt).  Here the states
+// costs three CTA barriers per step and four different instruction streams per CTA: the profiler shows `no_instruction`
+// and `barrier` as the first two stalls of such a kernel (profiles/r1_v19_decodeSplit_s159_ncu_full.txt).  Here the states
 // are cut across the LANES of a warp instead: a warp decodes 8 pairs, lane = (quarter g of the state range, pair p), so
 //   * every lane runs the same instructions (one body for the whole kernel: the sweeps stream from the instruction cache),
 //   * the four quarters of a scan meet through warp shuffles, not through shared memory and barriers,

@@ -1,36 +1,33 @@
 // fastsmc_b200 — lane-split decode kernel (decode_lane.cuh) for the 159-state decoding quantities (FASTSMC_EXAMPLE).
-#include <cstdlib>
-
 #include "decode_lane.cuh"
-#include "split_select.h"
+#include "lane_select.h"
 
 namespace fsmc
 {
 
 constexpr int kLaneGroup = 4, kLaneDepth = 2;
 
-template <int S, int RQ, int MINB> static SplitChoice makeLane()
+template <int S, int RQ, int MINB> static LaneChoice makeLane()
 {
-  return SplitChoice{decodeLaneKernel<S, RQ, kLaneGroup, kLaneDepth, MINB>, kLaneQuarters,
-                     LaneSmem<S, RQ, kLaneGroup, kLaneDepth>::kTotal, RQ, LaneGeom<S>::Spad, false};
+  return LaneChoice{decodeLaneKernel<S, RQ, kLaneGroup, kLaneDepth, MINB>, kLaneQuarters,
+                    LaneSmem<S, RQ, kLaneGroup, kLaneDepth>::kTotal, RQ, LaneGeom<S>::Spad};
 }
 
-template <int S, int MINB> static SplitChoice makeLaneWide()
+template <int S, int MINB> static LaneChoice makeLaneWide()
 {
-  return SplitChoice{decodeLaneWideKernel<S, kLaneGroup, kLaneDepth, MINB>, kLaneQuarters,
-                     LaneWideSmem<S, kLaneGroup, kLaneDepth>::kTotal, 0, LaneGeom<S>::Spad, true};
+  return LaneChoice{decodeLaneWideKernel<S, kLaneGroup, kLaneDepth, MINB>, kLaneQuarters,
+                    LaneWideSmem<S, kLaneGroup, kLaneDepth>::kTotal, 0, LaneGeom<S>::Spad};
 }
 
-SplitChoice laneKernel159(const int recordQuads)
+LaneChoice laneKernel159(const int recordQuads)
 {
-  static const bool four = [] { const char* e = std::getenv("FSMC_LANE"); return e && *e == '4'; }();  // A/B: 4 CTAs per SM (spills)
   switch (recordQuads) {
   case 0:
     return makeLaneWide<159, 3>();  // every state reaches the consumers: full beta rows through HBM
   case 1:
-    return four ? makeLane<159, 1, 4>() : makeLane<159, 1, 3>();
+    return makeLane<159, 1, 3>();
   case 2:
-    return four ? makeLane<159, 2, 4>() : makeLane<159, 2, 3>();
+    return makeLane<159, 2, 3>();
   case 3:
     return makeLane<159, 3, 3>();  // --time up to 140 generations with the example table
   case 4:

@@ -112,7 +112,7 @@ int fsmc_set_haplotypes(fsmc_ctx* ctx, const uint64_t* bits, int64_t numHaps, in
                                   /* results are bit-identical to the reference's NO_SSE build    */
 #define FSMC_GENERIC_KERNEL 0x40u /* force the any-S shared-memory kernel (testing)               */
 #define FSMC_WIDE_KERNEL 0x80u    /* never use the narrow (no beta round trip) kernel (testing)   */
-#define FSMC_ONE_WARP_KERNEL 0x100u /* never use the state-split kernels (one tile per CTA) (testing) */
+#define FSMC_ONE_WARP_KERNEL 0x100u /* never use the lane-split kernels (one tile per CTA) (testing)  */
 #define FSMC_SITE_POSTERIOR 0x200u /* full per-site posterior of every pair (HMM.cpp:1372-1389, ASMC::decodePairs
                                       per_pair_posteriors; HMM::decode)                             */
 #define FSMC_SUM_POSTERIOR 0x400u  /* per-site posterior summed over the real pairs of the call
@@ -168,7 +168,7 @@ typedef struct fsmc_decode_stats {
   int32_t statesKernel; /* S the kernel was specialised for, 0 = generic                          */
   int64_t scratchBytes; /* backward-sweep scratch in HBM                                          */
   int32_t narrowKernel; /* 1 if the kernel without the beta round trip ran (states < threshold only) */
-  int32_t tileWarps;    /* warps that shared a tile: 1, or 2 / 4 for the state-split kernels                */
+  int32_t tileWarps;    /* warps that shared a tile: 1, or 4 for the lane-split kernels                     */
   /* all-state age estimates without the beta round trip (csrc/decode_sparse.cuh): narrow sweeps + checkpoints, then
    * full posteriors only inside the IBD runs                                                                        */
   int32_t sparseKernel;     /* 1 if that path ran                                                  */

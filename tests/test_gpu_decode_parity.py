@@ -205,14 +205,14 @@ def synthetic69(oracle_mod, tmp_path_factory):
     return o, ctx
 
 
-@pytest.fixture(params=[0, 1], ids=["one-warp", "split"])
-def split(request, monkeypatch):
-    """FSMC_SPLIT selects the kernel family: 0 = one warp per tile (decode_fast.cuh), 1 = state-split (decode_split.cuh)."""
-    monkeypatch.setenv("FSMC_SPLIT", str(request.param))
-    return request.param
+@pytest.fixture(params=[False, True], ids=["default", "one-warp"])
+def one_warp(request):
+    """Extra decode flags: none, or FSMC_ONE_WARP_KERNEL.  At 69 states both run one warp per tile (decode_fast.cuh)."""
+    from fastsmc_b200 import _native as N
+    return N.ONE_WARP_KERNEL if request.param else 0
 
 
-def test_fast_kernel_per_site_outputs_69_states(synthetic69, split):
+def test_fast_kernel_per_site_outputs_69_states(synthetic69, one_warp):
     """Production kernel (FMA, rescaling every 4th site, bulk-copy ring): per-site posterior mean, IBD probability and MAP
     within the north-star tolerance of the oracle; ragged windows and a partially filled tile included."""
     from fastsmc_b200 import _native as N
@@ -223,15 +223,15 @@ def test_fast_kernel_per_site_outputs_69_states(synthetic69, split):
         mean, mp, ibd = o.decode_summary(a, b, frm, to)
         nb = (len(a) + 31) // 32
         tiles = ctx.make_tiles(a, b, windows=[[frm, to]] * nb, sites=o.sites)
-        r = ctx.decode(tiles, N.SITE_MEAN | N.SITE_MAP | N.SITE_IBD)
-        assert r.stats.statesKernel == 69 and r.stats.tileWarps == (2 if split else 1)
+        r = ctx.decode(tiles, N.SITE_MEAN | N.SITE_MAP | N.SITE_IBD | one_warp)
+        assert r.stats.statesKernel == 69 and r.stats.tileWarps == 1
         rows = tiles["rows"]
         np.testing.assert_allclose(r.site_mean[rows, :to - frm], mean, rtol=REL_TOL)
         np.testing.assert_allclose(r.site_ibd[rows, :to - frm], ibd, rtol=REL_TOL, atol=1e-12)
         assert (r.site_map[rows, :to - frm] != mp).mean() < 2e-3
 
 
-def test_fast_kernel_segments_69_states(synthetic69, tmp_path, split):
+def test_fast_kernel_segments_69_states(synthetic69, tmp_path, one_warp):
     """Whole all-pairs job slice through the production kernel vs the oracle: same segments (a boundary may move only
     where the IBD probability is within tolerance of a threshold), sums and age estimates within 1e-4."""
     from fastsmc_b200 import _native as N
@@ -249,9 +249,9 @@ def test_fast_kernel_segments_69_states(synthetic69, tmp_path, split):
         a.append(2 * i)
         b.append(2 * i + 1)
     tiles = ctx.make_tiles(np.array(a), np.array(b), sites=o.sites)
-    r = ctx.decode(tiles, N.CALL_SEGMENTS | N.SEG_AGE, segment_capacity=1 << 20)
+    r = ctx.decode(tiles, N.CALL_SEGMENTS | N.SEG_AGE | one_warp, segment_capacity=1 << 20)
     seg = r.segments
-    assert r.stats.statesKernel == 69 and r.stats.tileWarps == (2 if split else 1)
+    assert r.stats.statesKernel == 69 and r.stats.tileWarps == 1
     want = {(int(i[0]) * 32 + int(i[1]), int(i[4]), int(i[5])): f for i, f in zip(ints, floats)}
     got = {(int(s["pair"]), int(s["posStart"]), int(s["posEnd"])): s for s in seg}
     common = set(want) & set(got)
@@ -287,7 +287,7 @@ def test_segment_records_do_not_depend_on_previous_buffer_contents(synthetic69):
     assert (np.diff(key) > 0).all()  # sorted by (pair, start), every record once
 
 
-def test_narrow_kernel_matches_oracle_and_wide_kernel(oracle_mod, synthetic69, split):
+def test_narrow_kernel_matches_oracle_and_wide_kernel(oracle_mod, synthetic69, one_warp):
     """FastSMC's default flags (age estimates conditional on TMRCA < time): the kernel that keeps only the states below
     the threshold and carries the normaliser by the scale-factor recurrence (decodeNarrowKernel) gives the oracle's
     segments and per-site IBD probabilities within 1e-4, over a 3 000-site window (750 rescalings)."""
@@ -305,12 +305,12 @@ def test_narrow_kernel_matches_oracle_and_wide_kernel(oracle_mod, synthetic69, s
     # per-site IBD probability
     mean, mp, ibd = o.decode_summary(a, b, 0, o.sites, mean=False, map_=False)
     tiles = ctx.make_tiles(a, b, windows=[[0, o.sites]] * 3, sites=o.sites)
-    r = ctx.decode(tiles, N.SITE_IBD)
-    assert r.stats.narrowKernel == 1 and r.stats.tileWarps == (2 if split else 1)
+    r = ctx.decode(tiles, N.SITE_IBD | one_warp)
+    assert r.stats.narrowKernel == 1 and r.stats.tileWarps == 1
     np.testing.assert_allclose(r.site_ibd[tiles["rows"]], ibd, rtol=REL_TOL, atol=1e-12)
     # segments with conditional age estimates: narrow vs the full-beta kernel (same arithmetic otherwise)
-    rn = ctx.decode(tiles, N.CALL_SEGMENTS | N.SEG_AGE)
-    rw = ctx.decode(tiles, N.CALL_SEGMENTS | N.SEG_AGE | N.WIDE_KERNEL)
+    rn = ctx.decode(tiles, N.CALL_SEGMENTS | N.SEG_AGE | one_warp)
+    rw = ctx.decode(tiles, N.CALL_SEGMENTS | N.SEG_AGE | N.WIDE_KERNEL | one_warp)
     assert rn.stats.narrowKernel == 1 and rw.stats.narrowKernel == 0
     key = lambda s: (int(s["pair"]), int(s["posStart"]), int(s["posEnd"]))
     gn, gw = {key(s): s for s in rn.segments}, {key(s): s for s in rw.segments}
@@ -321,7 +321,7 @@ def test_narrow_kernel_matches_oracle_and_wide_kernel(oracle_mod, synthetic69, s
     assert np.mean([gn[k]["mapState"] != gw[k]["mapState"] for k in common]) < 5e-3
 
 
-# ---- 159 states (FASTSMC_EXAMPLE table): the state-split kernels are the production path (4 warps per tile) ---------
+# ---- 159 states (FASTSMC_EXAMPLE table): the lane-split kernels are the production path (4 warps per tile) ----------
 
 
 @pytest.mark.parametrize("time", [50, 100, 140], ids=["time50-2quads", "time100-3quads", "time140-4quads"])

@@ -4,8 +4,8 @@ Every field must equal what ASMC.decodePairs returns for the same inputs, bit fo
 the device adds them with float atomics); the host path's results must be left alone; nothing but O(1) statistics may cross
 to the host.  The 69-state model runs through ASMC.decodePairs on the bundled ASMC example.  The bundled 159-state table only
 holds the rows FastSMC mode needs (tests/golden/make_fixtures.py), so an ASMC-mode object cannot be built on it: the
-159-state kernels (decodeLaneWideKernel, decodeSplitKernel<159>, decodeTilesKernel<159>) are held to fsmc_decode, the call
-behind ASMC.decodePairs, through the C ABI."""
+159-state kernels (decodeLaneWideKernel, decodeTilesKernel<159>) are held to fsmc_decode, the call behind ASMC.decodePairs,
+through the C ABI."""
 import os
 import subprocess
 import sys
@@ -21,12 +21,11 @@ torch = pytest.importorskip("torch")
 HERE = os.path.dirname(os.path.abspath(__file__))
 ALL = dict(per_pair_posteriors=True, sum_of_posteriors=True, per_pair_posterior_means=True, per_pair_MAPs=True)
 SITE = dict(per_pair_posterior_means=True, per_pair_MAPs=True)
-# name -> (data, decoding quantities, exactArithmetic, outputs, environment, sums bit-identical)
+# name -> (data, decoding quantities, exactArithmetic, outputs, sums bit-identical)
 CASES = {
-    "fast69": (ASMC_EXAMPLE, DQ_69, False, dict(SITE, sum_of_posteriors=True), {}, True),  # decodeFastKernel<SUM>
-    "exact69": (ASMC_EXAMPLE, DQ_69, True, ALL, {}, False),                                # decodeTilesKernel
-    "posteriors69": (ASMC_EXAMPLE, DQ_69, False, dict(per_pair_posteriors=True), {}, False),
-    "split69": (ASMC_EXAMPLE, DQ_69, False, SITE, {"FSMC_SPLIT": "1"}, False),             # decodeSplitKernel<69>
+    "fast69": (ASMC_EXAMPLE, DQ_69, False, dict(SITE, sum_of_posteriors=True), True),  # decodeFastKernel<SUM>
+    "exact69": (ASMC_EXAMPLE, DQ_69, True, ALL, False),                                # decodeTilesKernel
+    "posteriors69": (ASMC_EXAMPLE, DQ_69, False, dict(per_pair_posteriors=True), False),
 }
 
 
@@ -85,7 +84,7 @@ def _same(got, want, name, sums_exact):
 def check_case(case, n=150, ids=False):
     """decode_pairs_cuda on a non-default stream vs ASMC.decodePairs, every field; the host results stay untouched."""
     from fastsmc_b200.cuda_results import decode_pairs_cuda
-    root, dq, exact, outputs, _, sums_exact = CASES[case]
+    root, dq, exact, outputs, sums_exact = CASES[case]
     m = _asmc(root, dq, exact)
     a, b = _pairs(n, seed=n)
     want = _host(m, a, b, outputs)
@@ -109,18 +108,9 @@ def check_case(case, n=150, ids=False):
                               want["per_pair_posterior_means"].view(np.uint32))
 
 
-@pytest.mark.parametrize("case", [c for c in CASES if not CASES[c][4]])
+@pytest.mark.parametrize("case", list(CASES))
 def test_device_outputs_equal_decode_pairs(case):
     check_case(case)
-
-
-@pytest.mark.parametrize("case", [c for c in CASES if CASES[c][4]])
-def test_device_outputs_equal_decode_pairs_kernel_variants(case):
-    """Kernel selections read from the environment once per process: each runs in a process of its own."""
-    env = dict(os.environ, **CASES[case][4])
-    code = f"import sys; sys.path.insert(0, {HERE!r}); import test_gpu_device_outputs as t; t.check_case({case!r})"
-    r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
 
 
 def test_device_outputs_across_chunks():
@@ -165,14 +155,6 @@ C_ABI_CASES = [(69, w) for w in FLAG_SETS] + [(159, w) for w in ("mean_map", "su
 @pytest.mark.parametrize("states,which", C_ABI_CASES)
 def test_decode_device_same_kernel_and_values_as_decode(states, which):
     check_c_abi(states, which)
-
-
-def test_decode_device_state_split_159():
-    """FSMC_LANE=0: the 159-state model on decodeSplitKernel<159> instead of decodeLaneWideKernel (read once per process)."""
-    env = dict(os.environ, FSMC_LANE="0")
-    code = f"import sys; sys.path.insert(0, {HERE!r}); import test_gpu_device_outputs as t; t.check_c_abi(159, 'mean_map')"
-    r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
 
 
 def check_c_abi(states, which):

@@ -3,7 +3,7 @@
 
     compute-sanitizer --tool racecheck python tools/racecheck_probe.py
 
-The mbarrier / bulk-copy ring protocols (decode_fast.cuh, decode_split.cuh, decode_sparse.cuh) are what the tool checks;
+The mbarrier / bulk-copy ring protocols (decode_fast.cuh, decode_lane.cuh, decode_sparse.cuh) are what the tool checks;
 the probe only asserts that every kernel ran and produced segments.
 """
 import os
@@ -45,13 +45,10 @@ def main():
         synth.dataset(root, 320, 640, 2_000_000, 1, 99)
     rng = np.random.default_rng(1)
     n_pairs = 5 * 32 + 7
-    for label, r, dq, conditional, env in (
-            ("wide69", root, DQ69, False, {}), ("narrow69", root, DQ69, True, {}),
-            ("split-wide69", root, DQ69, False, {"FSMC_SPLIT": "1"}), ("split-narrow69", root, DQ69, True, {"FSMC_SPLIT": "1"}),
-            ("lane-wide159", EX, EX + ".decodingQuantities.gz", False, {}),
-            ("lane-narrow159", EX, EX + ".decodingQuantities.gz", True, {})):
-        for k, v in env.items():
-            os.environ[k] = v
+    for label, r, dq, conditional in (
+            ("wide69", root, DQ69, False), ("narrow69", root, DQ69, True),
+            ("lane-wide159", EX, EX + ".decodingQuantities.gz", False),
+            ("lane-narrow159", EX, EX + ".decodingQuantities.gz", True)):
         ctx, data = context(r, dq, conditional)
         H, L = data.hapBits.shape[0], min(data.sites, 640)
         a = rng.integers(0, H - 1, n_pairs).astype(np.uint32)
@@ -64,8 +61,6 @@ def main():
         print(label, "segments", len(res.segments), "narrow", res.stats.narrowKernel, "tileWarps", res.stats.tileWarps,
               "states", res.stats.statesKernel, "ibd finite", bool(np.isfinite(res2.site_ibd).all()), flush=True)
         ctx.close()
-        for k in env:
-            del os.environ[k]
 
 
 if __name__ == "__main__":
