@@ -79,6 +79,17 @@ class DeviceOutputs(C.Structure):
     ]
 
 
+class DeviceSegments(C.Structure):
+    _fields_ = [("offset", C.c_int64), ("capacity", C.c_int64)] + [(f, C.c_void_p) for f in (
+        "ind1_dev", "hap1_dev", "ind2_dev", "hap2_dev", "startSite_dev", "endSite_dev", "startBp_dev", "endBp_dev",
+        "lengthCm_dev", "score_dev", "postMean_dev", "mapTime_dev")]
+
+
+# the columns of fsmc_device_segments, in order, with their element types (int32 or float32)
+SEGMENT_COLUMNS = (("ind1", "int32"), ("hap1", "int32"), ("ind2", "int32"), ("hap2", "int32"), ("start_site", "int32"),
+                   ("end_site", "int32"), ("start_bp", "int32"), ("end_bp", "int32"), ("length_cm", "float32"),
+                   ("score", "float32"), ("post_mean", "float32"), ("map_time", "float32"))
+
 SEGMENT_DTYPE = np.dtype([
     ("pair", np.uint32), ("posStart", np.int32), ("posEnd", np.int32), ("prob", np.float32),
     ("postMean", np.float32), ("mapTime", np.float32), ("mapState", np.int32), ("level", np.int32),
@@ -88,7 +99,8 @@ EXPORTS = [
     "fsmc_last_error", "fsmc_version", "fsmc_device_count", "fsmc_ctx_create", "fsmc_ctx_destroy",
     "fsmc_ctx_set_stream", "fsmc_set_model", "fsmc_set_haplotypes", "fsmc_decode", "fsmc_plan_create",
     "fsmc_plan_launch", "fsmc_plan_collect", "fsmc_plan_destroy", "fsmc_seed", "fsmc_query_kernel",
-    "fsmc_decode_device", "fsmc_column_min_f32", "fsmc_column_min_i32",
+    "fsmc_decode_device", "fsmc_column_min_f32", "fsmc_column_min_i32", "fsmc_set_site_positions",
+    "fsmc_plan_collect_device", "fsmc_device_alloc", "fsmc_device_free", "fsmc_copy_device",
 ]
 
 _lib = None
@@ -114,6 +126,11 @@ def lib():
         L.fsmc_plan_collect.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Request), C.POINTER(Stats)]
         L.fsmc_plan_destroy.argtypes = [C.c_void_p, C.c_void_p]
         L.fsmc_decode_device.argtypes = [C.c_void_p, C.POINTER(Request), C.POINTER(DeviceOutputs), C.POINTER(Stats)]
+        L.fsmc_set_site_positions.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
+        L.fsmc_plan_collect_device.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(DeviceSegments), C.POINTER(Stats)]
+        L.fsmc_device_alloc.argtypes = [C.c_void_p, C.c_int64, C.POINTER(C.c_void_p)]
+        L.fsmc_device_free.argtypes = [C.c_void_p, C.c_void_p]
+        L.fsmc_copy_device.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
         for f in (L.fsmc_column_min_f32, L.fsmc_column_min_i32):
             f.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]
         _lib = L
@@ -310,6 +327,12 @@ class Context:
         _check(lib().fsmc_decode_device(self._h, C.byref(req), C.byref(out), C.byref(stats)))
         return stats
 
+    def set_site_positions(self, genetic_positions, physical_positions):
+        """fsmc_set_site_positions: Morgans and bp of every site of the model (after set_model)."""
+        g = _f32(genetic_positions)
+        bp = np.ascontiguousarray(physical_positions, dtype=np.int32)
+        _check(lib().fsmc_set_site_positions(self._h, _p(g), _p(bp), len(g)))
+
     def column_min(self, m, out_min, out_argmin):
         """fsmc_column_min_f32 / _i32 of a 2-D row-major device tensor (float32 or int32) on the context's stream."""
         if m.dim() != 2 or m.stride(1) != 1 or out_min.numel() < m.shape[1] or out_argmin.numel() < m.shape[1]:
@@ -339,6 +362,20 @@ class Plan:
         o = self._out
         seg = o["seg"][:stats.numSegments] if o["seg"] is not None else None
         return DecodeResult(seg, o["mean"], o["smap"], o["ibd"], stats, o["post"], o["psum"])
+
+    def collect_device(self, columns=None, offset=0, capacity=None):
+        """fsmc_plan_collect_device into `columns` (a dict of SEGMENT_COLUMNS names -> device tensors, or raw pointers;
+        None = count only).  Returns (rc, stats); FSMC_E_OVERFLOW is returned, not raised."""
+        stats = Stats()
+        if columns is None:
+            _check(lib().fsmc_plan_collect_device(self.ctx._h, self._h, None, C.byref(stats)))
+            return 0, stats
+        ptr = lambda t: None if t is None else (t if isinstance(t, int) else t.data_ptr())  # noqa: E731
+        if capacity is None:
+            capacity = min(int(t.numel()) for t in columns.values() if t is not None and not isinstance(t, int))
+        out = DeviceSegments(int(offset), int(capacity), *[ptr(columns.get(name)) for name, _ in SEGMENT_COLUMNS])
+        rc = _check(lib().fsmc_plan_collect_device(self.ctx._h, self._h, C.byref(out), C.byref(stats)), allow=(E_OVERFLOW,))
+        return rc, stats
 
     def close(self):
         if self._h:

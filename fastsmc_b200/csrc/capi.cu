@@ -176,6 +176,10 @@ struct fsmc_ctx {
   // once per context, not once per call (they and cudaMemGetInfo were 10-90 ms of a 300 ms fsmc_decode call)
   std::map<std::tuple<const void*, int, size_t>, int> occupancy;
   DevBuf<uint32_t> colMinPart;  // fsmc_column_min_*: per-chunk (value, row) of every column
+  // fsmc_set_site_positions: genetic (Morgans) and physical position of every site; positionSites = 0 until set
+  DevBuf<float> siteGen;
+  DevBuf<int32_t> siteBp;
+  long long positionSites = 0;
 };
 
 struct fsmc_plan {
@@ -477,6 +481,7 @@ int fsmc_set_model(fsmc_ctx* ctx, const fsmc_model* mdl)
     }
   }
   FSMC_CUDA(cudaSetDevice(ctx->device));
+  ctx->positionSites = 0;  // fsmc_set_site_positions belongs to the model
   const int Spad = (S + 3) / 4 * 4;
   cudaStream_t st = ctx->stream;
   auto setThresholds = [&](DeviceModel& dm) {
@@ -661,7 +666,7 @@ cudaError_t residentBlocks(fsmc_ctx* ctx, const void* fn, const int threads, con
 namespace
 {
 // memory of the context's device (cudaMalloc'd or managed), not host memory or another device's
-int checkDevicePtr(const fsmc_ctx* ctx, const void* p, const char* what)
+int checkDevicePtr(const fsmc_ctx* ctx, const void* p, const char* what, const char* fn = "fsmc_decode_device")
 {
   cudaPointerAttributes at{};
   const cudaError_t e = cudaPointerGetAttributes(&at, p);
@@ -670,10 +675,10 @@ int checkDevicePtr(const fsmc_ctx* ctx, const void* p, const char* what)
     return fail(FSMC_E_INVALID, "%s is not a CUDA pointer (%s)", what, cudaGetErrorString(e));
   }
   if (at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged) {
-    return fail(FSMC_E_INVALID, "fsmc_decode_device: %s is host memory, device memory of device %d is needed", what, ctx->device);
+    return fail(FSMC_E_INVALID, "%s: %s is host memory, device memory of device %d is needed", fn, what, ctx->device);
   }
   if (at.device != ctx->device) {
-    return fail(FSMC_E_INVALID, "fsmc_decode_device: %s is on device %d, the context on device %d", what, at.device, ctx->device);
+    return fail(FSMC_E_INVALID, "%s: %s is on device %d, the context on device %d", fn, what, at.device, ctx->device);
   }
   return FSMC_OK;
 }
@@ -1186,6 +1191,43 @@ int fsmc_plan_launch(fsmc_ctx* ctx, fsmc_plan* plan)
 namespace
 {
 void fillStats(fsmc_ctx* ctx, const fsmc_plan* plan, long long found, int64_t d2h, fsmc_decode_stats* stats);
+
+// Waits for a launched plan and reads its counters (segment count, tile queue head, sparse items).  A sparse plan with more
+// run pieces than item slots is run again with enough of them; with growSegments, so is a plan whose records did not fit
+// its record buffer.
+int waitForCounters(fsmc_ctx* ctx, fsmc_plan* plan, unsigned long long counters[4], const bool growSegments)
+{
+  cudaStream_t st = ctx->stream;
+  for (;;) {
+    if (plan->numTiles > 0) {
+      FSMC_CUDA(cudaMemcpyAsync(counters, plan->counters.p, (plan->sparse ? 4 : 2) * sizeof(unsigned long long),
+                                cudaMemcpyDeviceToHost, st));
+    }
+    FSMC_CUDA(cudaStreamSynchronize(st));
+    plan->itemsFound = static_cast<long long>(counters[2]);
+    const long long found = static_cast<long long>(counters[0]);
+    const bool moreItems = plan->sparse && plan->itemsFound > plan->itemCapacity;
+    const bool moreSegments = growSegments && found > plan->segmentCapacity;
+    if (!moreItems && !moreSegments) {
+      return FSMC_OK;
+    }
+    // more run pieces than item slots: run the request again with enough of them (the launch re-allocates)
+    if (plan->itemsFound >= 0x7ffffff0ll) {
+      return fail(FSMC_E_NOMEM, "fsmc_plan_collect: %lld run pieces in one request; decode fewer tiles per call", plan->itemsFound);
+    }
+    if (moreItems) {
+      plan->itemCapacity = std::min<long long>(plan->itemsFound + plan->itemsFound / 8 + 1024, 0x7ffffff0ll);
+    }
+    if (moreSegments) {
+      plan->segmentCapacity = found + found / 8 + 1024;
+      FSMC_CUDA(plan->segments.ensure(static_cast<size_t>(plan->segmentCapacity)));
+    }
+    const int rc = fsmc_plan_launch(ctx, plan);
+    if (rc != FSMC_OK) {
+      return rc;
+    }
+  }
+}
 }  // namespace
 
 int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request* out, fsmc_decode_stats* stats)
@@ -1200,25 +1242,9 @@ int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request*
   cudaStream_t st = ctx->stream;
   const unsigned flags = plan->flags;
   unsigned long long counters[4] = {0, 0, 0, 0};
-  for (;;) {
-    if (plan->numTiles > 0) {
-      FSMC_CUDA(cudaMemcpyAsync(counters, plan->counters.p, (plan->sparse ? 4 : 2) * sizeof(unsigned long long),
-                                cudaMemcpyDeviceToHost, st));
-    }
-    FSMC_CUDA(cudaStreamSynchronize(st));
-    plan->itemsFound = static_cast<long long>(counters[2]);
-    if (!plan->sparse || plan->itemsFound <= plan->itemCapacity) {
-      break;
-    }
-    // more run pieces than item slots: run the request again with enough of them (the launch re-allocates)
-    if (plan->itemsFound >= 0x7ffffff0ll) {
-      return fail(FSMC_E_NOMEM, "fsmc_plan_collect: %lld run pieces in one request; decode fewer tiles per call", plan->itemsFound);
-    }
-    plan->itemCapacity = std::min<long long>(plan->itemsFound + plan->itemsFound / 8 + 1024, 0x7ffffff0ll);
-    const int rc = fsmc_plan_launch(ctx, plan);
-    if (rc != FSMC_OK) {
-      return rc;
-    }
+  const int wrc = waitForCounters(ctx, plan, counters, false);
+  if (wrc != FSMC_OK) {
+    return wrc;
   }
   const long long found = static_cast<long long>(counters[0]);
   const long long stored = std::min<long long>(found, plan->segmentCapacity);
@@ -1348,6 +1374,139 @@ int fsmc_plan_destroy(fsmc_ctx* ctx, fsmc_plan* plan)
   return FSMC_OK;
 }
 
+int fsmc_set_site_positions(fsmc_ctx* ctx, const float* geneticPositions, const int32_t* physicalPositions, const int64_t sites)
+{
+  if (!ctx || !geneticPositions || !physicalPositions) {
+    return fail(FSMC_E_INVALID, "fsmc_set_site_positions: NULL argument");
+  }
+  if (!ctx->hasModel || sites != ctx->model.L) {
+    return fail(FSMC_E_STATE, "fsmc_set_site_positions: %lld sites, the model has %d (set the model first)",
+                static_cast<long long>(sites), ctx->hasModel ? ctx->model.L : 0);
+  }
+  FSMC_CUDA(cudaSetDevice(ctx->device));
+  FSMC_CUDA(ctx->siteGen.ensure(static_cast<size_t>(sites)));
+  FSMC_CUDA(ctx->siteBp.ensure(static_cast<size_t>(sites)));
+  FSMC_CUDA(cudaMemcpyAsync(ctx->siteGen.p, geneticPositions, sites * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  FSMC_CUDA(cudaMemcpyAsync(ctx->siteBp.p, physicalPositions, sites * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+  FSMC_CUDA(cudaStreamSynchronize(ctx->stream));  // the caller's arrays may go away
+  ctx->positionSites = sites;
+  return FSMC_OK;
+}
+
+int fsmc_plan_collect_device(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_device_segments* out, fsmc_decode_stats* stats)
+{
+  if (!ctx || !plan) {
+    return fail(FSMC_E_INVALID, "fsmc_plan_collect_device: NULL argument");
+  }
+  if (!plan->launched) {
+    return fail(FSMC_E_STATE, "fsmc_plan_collect_device: plan was not launched");
+  }
+  if (!(plan->flags & FSMC_CALL_SEGMENTS)) {
+    return fail(FSMC_E_INVALID, "fsmc_plan_collect_device: the plan does not call segments (FSMC_CALL_SEGMENTS)");
+  }
+  if (ctx->positionSites != ctx->model.L) {
+    return fail(FSMC_E_STATE, "fsmc_plan_collect_device: set the site positions of the model first (fsmc_set_site_positions)");
+  }
+  if (out) {
+    if (out->offset < 0 || out->capacity < 0) {
+      return fail(FSMC_E_INVALID, "fsmc_plan_collect_device: offset=%lld capacity=%lld", static_cast<long long>(out->offset),
+                  static_cast<long long>(out->capacity));
+    }
+    const struct {
+      const void* p;
+      const char* name;
+      bool required;
+    } cols[] = {{out->ind1_dev, "ind1_dev", true},       {out->hap1_dev, "hap1_dev", true},
+                {out->ind2_dev, "ind2_dev", true},       {out->hap2_dev, "hap2_dev", true},
+                {out->startSite_dev, "startSite_dev", true}, {out->endSite_dev, "endSite_dev", true},
+                {out->startBp_dev, "startBp_dev", true}, {out->endBp_dev, "endBp_dev", true},
+                {out->lengthCm_dev, "lengthCm_dev", true}, {out->score_dev, "score_dev", true},
+                {out->postMean_dev, "postMean_dev", false}, {out->mapTime_dev, "mapTime_dev", false}};
+    for (const auto& c : cols) {
+      if (!c.p) {
+        if (c.required) {
+          return fail(FSMC_E_INVALID, "fsmc_plan_collect_device: %s is NULL", c.name);
+        }
+        continue;
+      }
+      const int rc = checkDevicePtr(ctx, c.p, c.name, "fsmc_plan_collect_device");
+      if (rc != FSMC_OK) {
+        return rc;
+      }
+    }
+  }
+  FSMC_CUDA(cudaSetDevice(ctx->device));
+  unsigned long long counters[4] = {0, 0, 0, 0};
+  int rc = waitForCounters(ctx, plan, counters, true);
+  if (rc != FSMC_OK) {
+    return rc;
+  }
+  const long long found = static_cast<long long>(counters[0]);
+  if (!out) {
+    fillStats(ctx, plan, found, 0, stats);
+    return FSMC_OK;
+  }
+  if (out->offset + found > out->capacity) {
+    fillStats(ctx, plan, found, 0, stats);
+    return fail(FSMC_E_OVERFLOW, "fsmc_plan_collect_device: %lld segments at offset %lld, capacity %lld", found,
+                static_cast<long long>(out->offset), static_cast<long long>(out->capacity));
+  }
+  cudaStream_t st = ctx->stream;
+  if (found > 0) {
+    // reference order = ascending (pair, first site), as in fsmc_plan_collect
+    const fsmc_segment* sorted = nullptr;
+    FSMC_CUDA(ctx->segmentSorter.sort(plan->segments.p, found, static_cast<uint32_t>(plan->numTiles * 32), st, &sorted));
+    FSMC_CUDA(fsmc::writeSegmentColumns(sorted, found, plan->hapA.p, plan->hapB.p, ctx->siteGen.p, ctx->siteBp.p, *out, st));
+  }
+  FSMC_CUDA(cudaEventRecord(ctx->ev[3], st));
+  FSMC_CUDA(cudaStreamSynchronize(st));
+  fillStats(ctx, plan, found, 0, stats);
+  plan->launched = false;
+  return FSMC_OK;
+}
+
+int fsmc_device_alloc(fsmc_ctx* ctx, const int64_t bytes, void** out_dev)
+{
+  if (!ctx || !out_dev || bytes < 0) {
+    return fail(FSMC_E_INVALID, "fsmc_device_alloc: NULL argument or negative size");
+  }
+  *out_dev = nullptr;
+  FSMC_CUDA(cudaSetDevice(ctx->device));
+  FSMC_CUDA(cudaMallocAsync(out_dev, static_cast<size_t>(std::max<int64_t>(bytes, 1)), ctx->stream));
+  return FSMC_OK;
+}
+
+int fsmc_device_free(fsmc_ctx* ctx, void* p_dev)
+{
+  if (!ctx) {
+    return fail(FSMC_E_INVALID, "fsmc_device_free: NULL context");
+  }
+  if (p_dev) {
+    FSMC_CUDA(cudaSetDevice(ctx->device));
+    FSMC_CUDA(cudaFreeAsync(p_dev, ctx->stream));
+  }
+  return FSMC_OK;
+}
+
+int fsmc_copy_device(fsmc_ctx* ctx, void* dst_dev, const void* src_dev, const int64_t bytes)
+{
+  if (!ctx || bytes < 0 || (bytes > 0 && (!dst_dev || !src_dev))) {
+    return fail(FSMC_E_INVALID, "fsmc_copy_device: NULL argument or negative size");
+  }
+  if (bytes == 0) {
+    return FSMC_OK;
+  }
+  int rc = checkDevicePtr(ctx, dst_dev, "dst_dev", "fsmc_copy_device");
+  if (rc == FSMC_OK) {
+    rc = checkDevicePtr(ctx, src_dev, "src_dev", "fsmc_copy_device");
+  }
+  if (rc != FSMC_OK) {
+    return rc;
+  }
+  FSMC_CUDA(cudaSetDevice(ctx->device));
+  FSMC_CUDA(cudaMemcpyAsync(dst_dev, src_dev, static_cast<size_t>(bytes), cudaMemcpyDeviceToDevice, ctx->stream));
+  return FSMC_OK;
+}
 
 int fsmc_seed(fsmc_ctx* ctx, const fsmc_seed_params* sp, fsmc_match* out, const int64_t capacity,
               fsmc_seed_stats* stats)

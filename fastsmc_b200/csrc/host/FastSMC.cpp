@@ -45,6 +45,12 @@ void ASMC::FastSMC::run()
             << " IBD segments detected." << std::endl;
 }
 
+void ASMC::FastSMC::runDeviceSegments()
+{
+  mHmm.setDeviceSegments(true);
+  run();
+}
+
 // ref: FastSMC.cpp:53-235.  The reference streams the haps file a second time, filling a ring of 64-SNP words per
 // haplotype and updating two hash maps word by word.  Here the packed haplotypes are already on the device; one
 // fsmc_seed call returns every match interval of the job.

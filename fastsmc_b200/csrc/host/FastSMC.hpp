@@ -27,6 +27,9 @@ public:
   /// Seeding (when hashing is on) -> batched decoding -> IBD segments written to
   /// <outFileRoot>.<jobInd>.<jobs>.FastSMC.{ibd,bibd}.gz (ref: FastSMC.cpp:41-238).
   void run();
+  /// What run() does, with the segments left on the device (HMM::setDeviceSegments) instead of written to a file: same
+  /// seeding, candidate order, chunks and records, in the file's order.  HMM::moveDeviceSegments hands them over.
+  void runDeviceSegments();
 
   // ---- B200 build: introspection -------------------------------------------------------------------------------
   struct SeedingStats {

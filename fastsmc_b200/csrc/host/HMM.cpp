@@ -396,7 +396,9 @@ void HMM::openOutput(const int jobs, const int jobInd)
 void HMM::decodeAll(const int jobs, const int jobInd)
 {
   if (decodingParams.FastSMC) {
-    openOutput(jobs, jobInd);
+    if (!m_deviceSegments) {
+      openOutput(jobs, jobInd);
+    }
     if (decodingParams.hashing) {
       return;
     }
@@ -642,6 +644,15 @@ struct HMM::ChunkJob {
   std::shared_ptr<SegmentBlock> block;
   fsmc_decode_stats st{};
   double decodeWallS = 0.0;
+  // device-segment mode: the launched plan, collected by completeChunk
+  fsmc_ctx* ctx = nullptr;
+  fsmc_plan* plan = nullptr;
+  ~ChunkJob()
+  {
+    if (plan) {
+      fsmc_plan_destroy(ctx, plan);
+    }
+  }
 };
 
 struct HMM::DecodePipeline {
@@ -667,6 +678,7 @@ HMM::~HMM()
       w.join();
     }
   }
+  releaseDeviceSegments(m_ctx);
   contextPool().release(decodingParams.device, m_ctx2);
   contextPool().release(decodingParams.device, m_ctx);
 }
@@ -687,6 +699,9 @@ void HMM::startDecodeWorkers()
   }
   if (workers == 2) {
     uploadModelTo(m_ctx2);
+    if (m_deviceSegments) {
+      uploadSitePositions();
+    }
   }
   for (int w = 0; w < workers; ++w) {
     fsmc_ctx* ctx = w == 0 ? m_ctx : m_ctx2;
@@ -788,20 +803,31 @@ void HMM::decodeChunk(ChunkJob& job, fsmc_ctx* ctx)
   // record buffer sized from the densest chunk seen so far (a retry after FSMC_E_OVERFLOW decodes the chunk again)
   size_t capacity =
       std::max<size_t>(1024, static_cast<size_t>(static_cast<double>(n) * m_segmentsPerPair.load() * 1.5) + 1024);
-  job.block = std::make_shared<SegmentBlock>();
-  for (;;) {
-    job.block->seg.reset(new fsmc_segment[capacity]);
-    req.segments = job.block->seg.get();
+  if (m_deviceSegments) {
+    // the records stay in the plan's device buffer (grown by the library if they do not fit) until completeChunk
     req.segmentCapacity = static_cast<int64_t>(capacity);
+    job.ctx = ctx;
     const double t0 = now();
-    const int rc = fsmc_decode(ctx, &req, &job.st);
+    check(fsmc_plan_create(ctx, &req, &job.plan), "fsmc_plan_create");
+    check(fsmc_plan_launch(ctx, job.plan), "fsmc_plan_launch");
+    check(fsmc_plan_collect_device(ctx, job.plan, nullptr, &job.st), "fsmc_plan_collect_device");  // the count
     job.decodeWallS += now() - t0;
-    if (rc == FSMC_E_OVERFLOW) {
-      capacity = static_cast<size_t>(job.st.numSegments) + 1024;
-      continue;
+  } else {
+    job.block = std::make_shared<SegmentBlock>();
+    for (;;) {
+      job.block->seg.reset(new fsmc_segment[capacity]);
+      req.segments = job.block->seg.get();
+      req.segmentCapacity = static_cast<int64_t>(capacity);
+      const double t0 = now();
+      const int rc = fsmc_decode(ctx, &req, &job.st);
+      job.decodeWallS += now() - t0;
+      if (rc == FSMC_E_OVERFLOW) {
+        capacity = static_cast<size_t>(job.st.numSegments) + 1024;
+        continue;
+      }
+      check(rc, "fsmc_decode");
+      break;
     }
-    check(rc, "fsmc_decode");
-    break;
   }
   const double perPair = static_cast<double>(job.st.numSegments) / static_cast<double>(n);
   double seen = m_segmentsPerPair.load();
@@ -821,11 +847,17 @@ void HMM::completeChunk(ChunkJob& job)
   m_stats.pairSites += st.pairSites;
   m_stats.kernelMs += st.kernelMs;
   m_stats.deviceMs += st.totalMs;
+  m_stats.d2hBytes += static_cast<double>(st.d2hBytes);
 
   const double t1 = now();
   const size_t count = static_cast<size_t>(st.numSegments);
   nbSegmentsDetected += count;
   m_stats.segments += count;
+  if (m_deviceSegments) {
+    appendDeviceSegments(job);
+    m_stats.outputWallS += now() - t1;
+    return;
+  }
   std::shared_ptr<SegmentBlock> block = job.block;
   block->count = count;
   block->pend = std::move(job.pend);
@@ -845,6 +877,98 @@ void HMM::completeChunk(ChunkJob& job)
     }
   }
   m_stats.outputWallS += now() - t1;
+}
+
+void HMM::setDeviceSegments(const bool on)
+{
+  drainDecodes();
+  releaseDeviceSegments(m_ctx);
+  m_deviceSegments = on;
+  if (on) {
+    uploadSitePositions();
+  }
+}
+
+void HMM::uploadSitePositions()
+{
+  for (fsmc_ctx* ctx : {m_ctx, m_ctx2}) {
+    if (ctx) {
+      check(fsmc_set_site_positions(ctx, data.geneticPositions.data(), data.physicalPositions.data(), data.sites),
+            "fsmc_set_site_positions");
+    }
+  }
+}
+
+// Frees the device columns on ctx's stream.  Every use of them has completed: fsmc_plan_collect_device returns when its
+// records are written, and moveDeviceSegments frees on the stream of its copies.
+void HMM::releaseDeviceSegments(fsmc_ctx* ctx)
+{
+  for (void*& col : m_segCols) {
+    if (col && ctx) {
+      fsmc_device_free(ctx, col);
+    }
+    col = nullptr;
+  }
+  m_segCount = m_segCapacity = 0;
+}
+
+// Runs on a decode worker in submission order, so the records land in file order.  The two workers' collects never
+// overlap: each returns when its records are written, and completeChunk runs for one chunk at a time.  Growing the columns
+// (allocate, copy, free on this worker's stream) therefore comes after every write of the other worker, and the collect
+// below, on the same stream, after the growth.
+void HMM::appendDeviceSegments(ChunkJob& job)
+{
+  const int64_t count = job.st.numSegments;
+  const bool ages = decodingParams.doPerPairPosteriorMean || decodingParams.doPerPairMAP;
+  const int columns = ages ? kSegmentColumns : kSegmentColumns - 2;
+  if (m_segCount + count > m_segCapacity || !m_segCols[0]) {
+    const int64_t cap = std::max<int64_t>(m_segCount + count, 2 * m_segCapacity);
+    for (int c = 0; c < columns; ++c) {
+      void* p = nullptr;
+      check(fsmc_device_alloc(job.ctx, cap * 4, &p), "fsmc_device_alloc");
+      if (m_segCols[c]) {
+        check(fsmc_copy_device(job.ctx, p, m_segCols[c], m_segCount * 4), "fsmc_copy_device");
+        check(fsmc_device_free(job.ctx, m_segCols[c]), "fsmc_device_free");
+      }
+      m_segCols[c] = p;
+    }
+    m_segCapacity = cap;
+  }
+  fsmc_device_segments out{};
+  out.offset = m_segCount;
+  out.capacity = m_segCapacity;
+  int32_t** ints[8] = {&out.ind1_dev,      &out.hap1_dev,    &out.ind2_dev,    &out.hap2_dev,
+                       &out.startSite_dev, &out.endSite_dev, &out.startBp_dev, &out.endBp_dev};
+  for (int c = 0; c < 8; ++c) {
+    *ints[c] = static_cast<int32_t*>(m_segCols[c]);
+  }
+  out.lengthCm_dev = static_cast<float*>(m_segCols[8]);
+  out.score_dev = static_cast<float*>(m_segCols[9]);
+  out.postMean_dev = decodingParams.doPerPairPosteriorMean ? static_cast<float*>(m_segCols[10]) : nullptr;
+  out.mapTime_dev = decodingParams.doPerPairMAP ? static_cast<float*>(m_segCols[11]) : nullptr;
+  fsmc_decode_stats st{};
+  check(fsmc_plan_collect_device(job.ctx, job.plan, &out, &st), "fsmc_plan_collect_device");
+  m_segCount += count;
+}
+
+void HMM::moveDeviceSegments(void* const dst[kSegmentColumns], void* stream)
+{
+  drainDecodes();
+  check(fsmc_ctx_set_stream(m_ctx, stream), "fsmc_ctx_set_stream");
+  int rc = FSMC_OK;
+  for (int c = 0; c < kSegmentColumns && rc == FSMC_OK; ++c) {
+    if (dst[c] && m_segCols[c]) {
+      rc = fsmc_copy_device(m_ctx, dst[c], m_segCols[c], m_segCount * 4);
+    }
+  }
+  if (rc == FSMC_OK) {
+    releaseDeviceSegments(m_ctx);  // on `stream`, after the copies
+  }
+  const std::string err = rc == FSMC_OK ? "" : fsmc_last_error();
+  check(fsmc_ctx_set_stream(m_ctx, nullptr), "fsmc_ctx_set_stream");
+  if (rc != FSMC_OK) {
+    throw std::runtime_error("fsmc_copy_device: " + err);
+  }
 }
 
 IbdSegment HMM::toIbdSegment(const SegmentBlock& block, const size_t i) const

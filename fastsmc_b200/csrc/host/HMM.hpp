@@ -156,6 +156,17 @@ public:
   const RunStats& getRunStats() const { return m_stats; }
   fsmc_ctx* context() { return m_ctx; }
   int getDevice() const { return decodingParams.device; }  // CUDA device of the decode context
+  /// Device-segment mode: the segments of the run stay on the device, as the columns of fsmc_device_segments in the order
+  /// of the .ibd.gz file, and no output file is opened.  Chunks, decode workers and statistics are those of the file run.
+  void setDeviceSegments(bool on);
+  /// Columns of the device segments, in fsmc_device_segments order: ind1, hap1, ind2, hap2, startSite, endSite, startBp,
+  /// endBp (int32), lengthCm, score, postMean, mapTime (float).  The last two only with per-pair posterior means / MAPs.
+  static constexpr int kSegmentColumns = 12;
+  /// Copies the device segments of the run (getDeviceSegmentCount() records) into dst[c] (device memory of the decoding
+  /// device, NULL = column not wanted) on `stream` (cudaStream_t; NULL = the context's own stream) and releases the
+  /// columns, ordered after the copies on that stream.
+  void moveDeviceSegments(void* const dst[kSegmentColumns], void* stream);
+  int64_t getDeviceSegmentCount() const { return m_segCount; }
   /// segments of the run are also kept in memory when this is set (tests, Python callers)
   void setKeepSegments(bool keep) { m_keepSegments = keep; }
   const std::vector<IbdSegment>& getSegments() const { return m_segments; }
@@ -204,6 +215,9 @@ private:
   RunStats m_stats;
   bool m_keepSegments = false;
   std::vector<IbdSegment> m_segments;
+  bool m_deviceSegments = false;
+  void* m_segCols[kSegmentColumns] = {};  // device columns of the device-segment mode (4-byte elements)
+  int64_t m_segCount = 0, m_segCapacity = 0;
 
   void uploadModel();
   void uploadModelTo(fsmc_ctx*& ctx);
@@ -211,6 +225,9 @@ private:
   void drainDecodes();
   void decodeChunk(ChunkJob& job, fsmc_ctx* ctx);
   void completeChunk(ChunkJob& job);
+  void appendDeviceSegments(ChunkJob& job);
+  void uploadSitePositions();
+  void releaseDeviceSegments(fsmc_ctx* ctx);
   void openOutput(int jobs, int jobInd);
   void flushPending(bool all);
   void runSegmentChunk(const Pending* pairs, size_t n);

@@ -323,6 +323,23 @@ PYBIND11_MODULE(pyASMC, m)
       .def("getRunStats", &HMM::getRunStats, py::return_value_policy::reference_internal)
       .def("getNumberOfDetectedSegments", &HMM::getNumberOfDetectedSegments)
       .def("getDevice", &HMM::getDevice)
+      .def("getDeviceSegmentCount", &HMM::getDeviceSegmentCount)
+      // raw device pointers (e.g. torch's data_ptr()) of the kSegmentColumns columns, 0 = not wanted, and a cudaStream_t
+      // as an integer; fastsmc_b200.cuda_results.fastsmc_segments_cuda allocates the tensors
+      .def(
+          "moveDeviceSegments",
+          [](HMM& self, const std::vector<uintptr_t>& dst, const uintptr_t stream) {
+            if (dst.size() != HMM::kSegmentColumns) {
+              throw std::runtime_error("moveDeviceSegments: one pointer per column (" + std::to_string(HMM::kSegmentColumns) + ")");
+            }
+            void* p[HMM::kSegmentColumns];
+            for (int c = 0; c < HMM::kSegmentColumns; ++c) {
+              p[c] = reinterpret_cast<void*>(dst[c]);
+            }
+            py::gil_scoped_release release;
+            self.moveDeviceSegments(p, reinterpret_cast<void*>(stream));
+          },
+          "dst"_a, "stream"_a = 0)
       .def("getModelTables", [](const HMM& h) { return tablesToDict(h.getModelTables(), h.getDecodingQuantities()); });
 
 
@@ -352,6 +369,7 @@ PYBIND11_MODULE(pyASMC, m)
       .def(py::init<const std::string&, const std::string&>(), "in_dir"_a, "out_dir"_a)
       .def(py::init<DecodingParams, Data>(), "decodingParams"_a, "data"_a)
       .def("run", &ASMC::FastSMC::run, py::call_guard<py::gil_scoped_release>())
+      .def("runDeviceSegments", &ASMC::FastSMC::runDeviceSegments, py::call_guard<py::gil_scoped_release>())
       .def("getSeedingStats", &ASMC::FastSMC::getSeedingStats, py::return_value_policy::reference_internal)
       .def("setKeepCandidates", &ASMC::FastSMC::setKeepCandidates)
       .def("getCandidates",

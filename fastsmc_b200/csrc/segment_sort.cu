@@ -31,7 +31,48 @@ __global__ void segmentGatherKernel(const fsmc_segment* __restrict__ in, const u
     dst[i] = src[2ll * index[i >> 1] + (i & 1)];
   }
 }
+
+// HMM::toIbdSegment + the fields of HMM::formatSegments, one record per thread, with the writer's roundings
+__global__ void segmentColumnsKernel(const fsmc_segment* __restrict__ in, const long long n, const uint32_t* __restrict__ hapA,
+                                     const uint32_t* __restrict__ hapB, const float* __restrict__ gen,
+                                     const int32_t* __restrict__ bp, const fsmc_device_segments out)
+{
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const fsmc_segment g = in[i];
+    const uint32_t a = hapA[g.pair], b = hapB[g.pair];
+    const long long o = out.offset + i;
+    out.ind1_dev[o] = static_cast<int32_t>(a / 2);
+    out.hap1_dev[o] = 1 + static_cast<int32_t>(a % 2);
+    out.ind2_dev[o] = static_cast<int32_t>(b / 2);
+    out.hap2_dev[o] = 1 + static_cast<int32_t>(b % 2);
+    out.startSite_dev[o] = g.posStart;
+    out.endSite_dev[o] = g.posEnd;
+    out.startBp_dev[o] = bp[g.posStart];
+    out.endBp_dev[o] = bp[g.posEnd];
+    out.lengthCm_dev[o] = __fmul_rn(100.f, __fsub_rn(gen[g.posEnd], gen[g.posStart]));
+    const double sites = static_cast<double>(static_cast<unsigned>(g.posEnd - g.posStart) + 1u);
+    out.score_dev[o] = __double2float_rn(__ddiv_rn(static_cast<double>(g.prob), sites));
+    if (out.postMean_dev) {
+      out.postMean_dev[o] = g.postMean;
+    }
+    if (out.mapTime_dev) {
+      out.mapTime_dev[o] = g.mapTime;
+    }
+  }
+}
 }  // namespace
+
+cudaError_t writeSegmentColumns(const fsmc_segment* sorted, const long long n, const uint32_t* hapA, const uint32_t* hapB,
+                                const float* gen, const int32_t* bp, const fsmc_device_segments& out, cudaStream_t stream)
+{
+  if (n <= 0) {
+    return cudaSuccess;
+  }
+  const int blocks = static_cast<int>(std::min<long long>((n + 255) / 256, 148 * 8));
+  segmentColumnsKernel<<<blocks, 256, 0, stream>>>(sorted, n, hapA, hapB, gen, bp, out);
+  return cudaGetLastError();
+}
 
 SegmentSorter::~SegmentSorter()
 {

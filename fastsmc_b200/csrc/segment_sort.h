@@ -37,4 +37,9 @@ private:
   size_t mCapacity = 0;
 };
 
+// The columns of fsmc_plan_collect_device from n sorted records: record i goes to index out.offset + i.  hapA / hapB are
+// the plan's haplotypes per pair (tile * 32 + lane); gen / bp the site positions.
+cudaError_t writeSegmentColumns(const fsmc_segment* sorted, long long n, const uint32_t* hapA, const uint32_t* hapB,
+                                const float* gen, const int32_t* bp, const fsmc_device_segments& out, cudaStream_t stream);
+
 }  // namespace fsmc

@@ -1,7 +1,10 @@
-"""ASMC.decodePairs results as CUDA tensors, written in place by the decode kernels.
+"""ASMC.decodePairs results and FastSMC's IBD segments as CUDA tensors, built on the device.
 
     res = decode_pairs_cuda(asmc_obj, haps_a, haps_b, per_pair_posterior_means=True)
     res.per_pair_posterior_means   # torch.float32 [pairs][sites] on cuda:{params.device}
+
+    seg = fastsmc_segments_cuda(params)
+    seg.ind1, seg.start_bp, seg.score  # one tensor per field of the .ibd.gz records, in the file's order
 
 The fields carry the names of the reference's DecodePairsReturnStruct and the values ASMC.decodePairs returns, bit for bit
 (the sums of posteriors to float rounding where the device adds them with atomics).  Nothing but O(1) statistics crosses
@@ -107,4 +110,56 @@ def decode_pairs_cuda(asmc, haps_a, haps_b, *, per_pair_posteriors=False, sum_of
                     ctx.column_min(res.per_pair_MAPs, res.min_MAPs, res.argmin_MAPs)
             finally:
                 ctx.set_stream(None)
+    return res
+
+
+_CUDA_STREAM_LEGACY = 0x1  # cudaStreamLegacy (cuda_runtime_api.h): the legacy default stream
+
+
+class FastSMCSegmentsCuda:
+    """The IBD segments of one FastSMC run as CUDA tensors of n_segments records each, in the order of the run's .ibd.gz /
+    .bibd.gz.  post_mean / map_time are None unless doPerPairPosteriorMean / doPerPairMAP are set."""
+
+    def __init__(self):
+        self.n_segments = 0
+        self.ind1 = self.hap1 = self.ind2 = self.hap2 = None  # int32: index into fam_ids / iids, haplotype 1 or 2
+        self.start_site = self.end_site = None               # int32, end inclusive
+        self.start_bp = self.end_bp = None                   # int32
+        self.length_cm = self.score = None                   # float32: 100 * (gen[end] - gen[start]); prob / sites
+        self.post_mean = self.map_time = None                # float32 or None
+        self.fam_ids = []
+        self.iids = []
+        self.d2h_bytes = 0                                   # decode outputs copied device -> host during the call (0)
+        self.decode_kernel_ms = 0.0                          # device time of the decode kernels (CUDA events)
+
+
+def fastsmc_segments_cuda(params, data=None):
+    """What FastSMC(params).run() computes (seeding, candidate order and decoding, with or without hashing, for the job
+    jobInd of jobs), with the segments returned as tensors on cuda:{params.device} instead of written to a file.  No file is
+    created.  The tensors are written on torch.cuda.current_stream().  `data`: an asmc.Data already loaded for params, as
+    FastSMC(params, data) takes it."""
+    from . import asmc
+    f = asmc.FastSMC(params) if data is None else asmc.FastSMC(params, data)
+    f.runDeviceSegments()
+    hmm = f.hmm()
+    n = int(hmm.getDeviceSegmentCount())
+    dev = torch.device("cuda", hmm.getDevice())
+    res = FastSMCSegmentsCuda()
+    res.n_segments = n
+    data = f.data()
+    res.fam_ids, res.iids = list(data.FamIDList), list(data.IIDList)
+    res.d2h_bytes = int(hmm.getRunStats().d2hBytes)
+    res.decode_kernel_ms = float(hmm.getRunStats().kernelMs)
+    wanted = {"post_mean": params.doPerPairPosteriorMean, "map_time": params.doPerPairMAP}
+    with torch.cuda.device(dev):
+        stream = torch.cuda.current_stream(dev)
+        dst = []
+        for name, dtype in _native.SEGMENT_COLUMNS:
+            t = torch.empty(n, dtype=getattr(torch, dtype), device=dev) if wanted.get(name, True) else None
+            setattr(res, name, t)
+            dst.append(t.data_ptr() if t is not None and n > 0 else 0)
+        # the decode workers' collects have completed when runDeviceSegments returns: the copies only need to follow
+        # torch's earlier work on its stream, which they do by running on it.  torch's default stream has the handle 0,
+        # which the library reads as "the context's own stream": name it as cudaStreamLegacy instead.
+        hmm.moveDeviceSegments(dst, stream.cuda_stream or _CUDA_STREAM_LEGACY)
     return res

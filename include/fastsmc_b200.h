@@ -242,6 +242,55 @@ int fsmc_plan_launch(fsmc_ctx* ctx, fsmc_plan* plan);
 int fsmc_plan_collect(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_decode_request* out, fsmc_decode_stats* stats);
 int fsmc_plan_destroy(fsmc_ctx* ctx, fsmc_plan* plan);
 
+/* ------------------------------------------------------------------------------------------------
+ * Device-resident IBD segments: the records of a launched FSMC_CALL_SEGMENTS plan, put in the order of the .ibd.gz file
+ * and turned into the columns the file's writer prints (HMM::formatSegments), in caller-owned device memory of the
+ * context's device (e.g. torch tensors).  No record crosses to the host.
+ *
+ * fsmc_set_site_positions: the genetic (Morgans, Data::geneticPositions) and physical (bp) position of every site of the
+ * model, uploaded once per model.  fsmc_set_model forgets them.
+ *
+ * fsmc_plan_collect_device:
+ *   - waits for the plan's kernels and reads its record count (at most 32 bytes).  A plan whose record buffer
+ *     (segmentCapacity of its request) was too small is decoded again with a large enough one;
+ *   - out == NULL: only counts, stats->numSegments is set and the plan stays collectable;
+ *   - offset + count > capacity: FSMC_E_OVERFLOW with stats->numSegments = count; nothing is written and the plan stays
+ *     collectable, so the caller can grow its columns without decoding again;
+ *   - otherwise sorts the records like fsmc_plan_collect, then one kernel writes record i of the sorted order at index
+ *     offset + i of every column.  Pair p = tile * 32 + lane of the request is haplotypes hapA[p], hapB[p]: individual
+ *     h / 2, haplotype 1 + h % 2.  lengthCm = 100.f * (gen[end] - gen[start]) and score = float(prob / double(end - start
+ *     + 1)), with the writer's roundings.
+ * Every column pointer must be memory of the context's device.  The work runs on the context's stream and the call returns
+ * when it has completed.  stats->d2hBytes is 0.
+ * ------------------------------------------------------------------------------------------------ */
+int fsmc_set_site_positions(fsmc_ctx* ctx, const float* geneticPositions, const int32_t* physicalPositions, int64_t sites);
+
+typedef struct fsmc_device_segments {
+  int64_t offset;           /* index of the plan's first record in every column                              */
+  int64_t capacity;         /* records every column holds                                                    */
+  int32_t* ind1_dev;        /* individual of hapA (index into Data::FamIDList / IIDList)                      */
+  int32_t* hap1_dev;        /* 1 or 2                                                                         */
+  int32_t* ind2_dev;
+  int32_t* hap2_dev;
+  int32_t* startSite_dev;   /* first site of the segment                                                      */
+  int32_t* endSite_dev;     /* last site (inclusive)                                                          */
+  int32_t* startBp_dev;
+  int32_t* endBp_dev;
+  float* lengthCm_dev;
+  float* score_dev;
+  float* postMean_dev;      /* NULL = not written (needs FSMC_SEG_AGE to hold values)                          */
+  float* mapTime_dev;       /* NULL = not written                                                             */
+} fsmc_device_segments;
+int fsmc_plan_collect_device(fsmc_ctx* ctx, fsmc_plan* plan, const fsmc_device_segments* out, fsmc_decode_stats* stats);
+
+/* Device memory for callers that hold device-resident results without a CUDA runtime of their own (the host layer's
+ * segment columns).  Stream-ordered on the context's stream (cudaMallocAsync / cudaFreeAsync / cudaMemcpyAsync): memory
+ * that other streams used must be freed after that use has completed.  fsmc_copy_device copies `bytes` between two buffers
+ * of the context's device and returns without waiting.                                                                   */
+int fsmc_device_alloc(fsmc_ctx* ctx, int64_t bytes, void** out_dev);
+int fsmc_device_free(fsmc_ctx* ctx, void* p_dev);
+int fsmc_copy_device(fsmc_ctx* ctx, void* dst_dev, const void* src_dev, int64_t bytes);
+
 
 /* ------------------------------------------------------------------------------------------------
  * Seeding: replaces the GERMLINE-style candidate search of FastSMC::run (FastSMC.cpp:144-229):
